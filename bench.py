@@ -10,8 +10,11 @@ kernel) + mask-based partial reset + one forward pass + the (torch) MDP glue of
 ``VelocityFlatEnv.step``.  ``value`` uses device-resident actions; ``e2e`` feeds actions from pinned
 host memory and reads reward/done/obs back every step.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--envs E]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--envs E] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...      (one rank per GPU, weak scaling)
+
+``--dump-outputs DIR`` writes what the last timed env step returned (rank 0's envs) as float32 ``DIR/<name>.npy``,
+so that two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.
 """
 
 from __future__ import annotations
@@ -67,6 +70,30 @@ def make_env(workload: str, envs: int, seed: int, dev: str):
     return VelocityFlatEnv(VelocityEnvCfg(robot="go1", terrain="rough" if workload == "E" else "rough_hf",
                                           num_envs=envs, seed=seed), device=dev)
   return VelocityFlatEnv(VelocityEnvCfg(num_envs=envs, seed=seed), device=dev)
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, out) -> None:
+  """obs, reward, terminated, truncated and the extras' tensors of one env step, as float32 .npy files.  Above
+  DUMP_MAX_BYTES in all, a fixed seeded sample of env rows is written, with its indices as env_ids.npy."""
+  import numpy as np
+
+  obs, reward, terminated, truncated, extras = out
+  arrays = {"obs": obs, "reward": reward, "terminated": terminated, "truncated": truncated, **extras}
+  arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+  n = len(reward)
+  row_bytes = sum(a.nbytes for a in arrays.values()) // n
+  if row_bytes * n > DUMP_MAX_BYTES:
+    rows = (DUMP_MAX_BYTES - 128 * (len(arrays) + 1)) // (row_bytes + 8)  # (128: a .npy header)
+    ids = np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+    arrays = {k: a[ids] for k, a in arrays.items()}
+    arrays["env_ids"] = ids.astype(np.float64)
+  d = Path(out_dir)
+  d.mkdir(parents=True, exist_ok=True)
+  for k, a in arrays.items():
+    np.save(d / f"{k}.npy", a)
 
 
 def _peaks():
@@ -352,6 +379,7 @@ def main():
   ap.add_argument("--no-flush", action="store_true")
   ap.add_argument("--preroll", type=int, default=100, help="untimed env steps before warm-up")
   ap.add_argument("--no-graph", action="store_true", help="do not capture the env step in a CUDA graph")
+  ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
   args = ap.parse_args()
   if args.impl == "reference":
     return run_reference(args)
@@ -402,7 +430,8 @@ def main():
         action = host_actions[k].to(dev, non_blocking=True)
       else:
         action = torch.rand((n, nu), generator=gen, device=dev) * 2 - 1
-      obs, reward, terminated, truncated, _ = env.step(action)
+      out = env.step(action)
+      obs, reward, terminated, truncated, _ = out
       gather_logs(env.log_row)  # packed (reward, terminated, truncated), written by the env step itself
       if kind == "host":
         out_r.copy_(reward, non_blocking=True)
@@ -422,7 +451,8 @@ def main():
     j1.record()
     torch.cuda.synchronize()
     total = sum(a.elapsed_time(b) for a, b in ev) + j0.elapsed_time(j1)
-    return total, (n * nu * 4, n * 4 + n * 2 + (obs.numel() * 4)) if kind == "host" else None
+    # (with the CUDA graph the returned tensors are its static outputs: the next step overwrites them)
+    return total, (n * nu * 4, n * 4 + n * 2 + (obs.numel() * 4)) if kind == "host" else None, out
 
   def barrier():
     if world > 1:
@@ -476,10 +506,12 @@ def main():
   if rank == 0:
     sampler.start()
   wall0 = time.perf_counter()
-  total_ms, _ = run("device", K, True)
+  total_ms, _, out = run("device", K, True)
   barrier()
   wall = time.perf_counter() - wall0
   clocks = sampler.stop() if rank == 0 else None
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, out)
   launches = launches_per_step * K
   total_ms = maxr(total_ms)
   st = env.sim.stats()
@@ -490,7 +522,7 @@ def main():
   # ---- end-to-end through host buffers -----------------------------------------------------------
   run("host", W, False)
   barrier()
-  e2e_ms, (h2d, d2h) = run("host", K, True)
+  e2e_ms, (h2d, d2h), _ = run("host", K, True)
   barrier()
   e2e_ms = maxr(e2e_ms)
 

@@ -1,14 +1,18 @@
-"""Run test files of the reference (unmodified, where they lie under /root/reference/tests) against this repo's
-stand-ins: ``mujoco`` / ``mujoco_warp`` / ``warp`` from mjlab_b200.compat, ``mjlab`` from baseline/_ref (tests/refload.py),
+"""Run test files of the reference (unmodified, under oracle/_ref/tests) against this repo's
+stand-ins: ``mujoco`` / ``mujoco_warp`` / ``warp`` from mjlab_b200.compat, ``mjlab`` from oracle/_ref (tests/refload.py),
 and - there being no GPU in the container - the engine compiled for the host (tests/emul/engine.py) behind the
 ``mujoco_warp`` stand-in.  Used by tests/test_reference_own_tests.py:  python tests/ref_runner.py <pytest args>
 On a GPU box `B2_REF_DEVICE=cuda:0 python tests/ref_runner.py tests/ref_env_cases.py` runs the env cases on libb2sim.so
 (tools/gpu_round.sh does; not part of `-m gpu` until it has been seen green there)."""
+import os
 import sys
 from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
 sys.path[:0] = [str(HERE.parent), str(HERE), str(HERE / "emul"), str(HERE / "stubs")]  # stubs: prettytable stand-in
+if not os.environ.get("B2_REF_DEVICE", "cpu").startswith("cuda"):
+  # the host-emulated engine takes host tensors; the reference's tests pick cuda:0 whenever torch sees a GPU
+  os.environ["CUDA_VISIBLE_DEVICES"] = ""
 
 import mjlab_b200.compat as compat  # noqa: E402
 import refload  # noqa: E402
@@ -52,8 +56,6 @@ import mjlab_b200.compat.mujoco_warp_shim as mw  # noqa: E402
 from engine import EmulEngine  # noqa: E402
 from mjlab_b200.sim import native  # noqa: E402
 
-import os  # noqa: E402
-
 if not os.environ.get("B2_REF_DEVICE", "cpu").startswith("cuda"):  # (on a GPU box: the real engine, libb2sim.so)
   mw._Engine = EmulEngine
 
@@ -68,4 +70,5 @@ if not os.environ.get("B2_REF_DEVICE", "cpu").startswith("cuda"):
 
 import pytest  # noqa: E402
 
-sys.exit(pytest.main(["-q", "-c", "/dev/null", "-p", "no:cacheprovider", *sys.argv[1:]]))
+# confcutdir: collection starts at the repository, not at the filesystem root (whose directories may be unreadable)
+sys.exit(pytest.main(["-q", "-c", "/dev/null", "--confcutdir", str(HERE.parent), "-p", "no:cacheprovider", *sys.argv[1:]]))

@@ -1,4 +1,4 @@
-"""Load the reference's own modules (installed unmodified under baseline/_ref by tools/install_reference.py)
+"""Load the reference's own modules (installed unmodified under oracle/_ref by oracle/install_reference.py)
 on top of mjlab_b200.compat, for the drop-in tests.
 
 Only the packages whose ``__init__`` drags in viewers / RL / terrain tooling that the image lacks (viser,
@@ -15,7 +15,7 @@ import types
 from pathlib import Path
 
 ROOT = Path(__file__).resolve().parents[1]
-REF = ROOT / "baseline" / "_ref"
+REF = ROOT / "oracle" / "_ref"
 
 
 def available() -> bool:

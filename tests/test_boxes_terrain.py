@@ -133,7 +133,9 @@ def test_terrain_census_and_geometry():
 
 
 def _go1_on(cfg, threshold=None):
-  from mjlab_b200.asset_zoo import go1, reference_xml
+  from util import golden_xml
+
+  from mjlab_b200.asset_zoo import go1
 
   old = C.STATIC_GRID_THRESHOLD
   if threshold is not None:
@@ -142,7 +144,7 @@ def _go1_on(cfg, threshold=None):
     tsp, origins = terrain_spec(cfg)
     sp = S.Spec()
     sp.attach(tsp, prefix="")
-    sp.attach(go1.robot_cfg(reference_xml("go1"), go1.velocity_sensors()).build_spec(), prefix="robot/")
+    sp.attach(go1.robot_cfg(golden_xml("go1"), go1.velocity_sensors()).build_spec(), prefix="robot/")
     sp.option.timestep = 0.005
     sp.option.integrator = S.INT_IMPLICITFAST
     sp.option.iterations, sp.option.ls_iterations = 10, 20
@@ -160,10 +162,6 @@ def go1_stairs():
 
 
 def test_grid_broadphase_equals_exhaustive_pairs(go1_stairs):
-  from mjlab_b200.asset_zoo import _REF_ZOO
-
-  if not _REF_ZOO.exists():
-    pytest.skip("reference MJCF not available (authoring container only)")
   sys.path.insert(0, str(Path(__file__).resolve().parents[1] / "tools"))
   from compile_assets import SMALL_STAIRS
 

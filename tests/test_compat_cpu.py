@@ -1,5 +1,5 @@
 """Host-side logic of mjlab_b200.compat (no GPU): the stand-in modules register only when the real ones are
-absent, the reference's own sim-layer files import and run against them (baseline/_ref, unmodified), and the
+absent, the reference's own sim-layer files import and run against them (oracle/_ref, unmodified), and the
 pieces that need no engine — wp.array views, the vectorised wp.launch, TorchArray/WarpBridge over CPU tensors,
 the MjModel accessors and the entity spec view — behave as the reference code expects."""
 
@@ -11,7 +11,7 @@ import torch
 
 import refload
 
-pytestmark = pytest.mark.skipif(not refload.available(), reason="baseline/_ref not installed (tools/install_reference.py)")
+pytestmark = pytest.mark.skipif(not refload.available(), reason="oracle/_ref not installed (oracle/install_reference.py)")
 
 
 @pytest.fixture(scope="module")
@@ -25,7 +25,7 @@ def test_reference_modules_load_from_their_own_files(ref):
   for mod in (mujoco, mujoco_warp, warp):
     assert getattr(mod, "__b2_compat__", False) or mod.__name__ in ("mujoco", "mujoco_warp", "warp")
   assert ref.sim.Simulation.__module__ == "mjlab.sim.sim"
-  assert "baseline/_ref/mjlab/envs/mdp/events.py" in ref.events.__file__.replace("\\", "/")
+  assert "oracle/_ref/mjlab/envs/mdp/events.py" in ref.events.__file__.replace("\\", "/")
   assert mujoco.mjtJoint.mjJNT_FREE == 0 and mujoco.mjtGeom.mjGEOM_BOX == 6 and mujoco.mjtObj.mjOBJ_XBODY == 2
 
 

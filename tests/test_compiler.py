@@ -183,13 +183,12 @@ def test_compiled_blobs_are_reproducible_from_the_reference_xml():
   compiler produces today from the reference's MJCF: arrays, names and keyframes, bit for bit."""
   import sys
 
-  from mjlab_b200.asset_zoo import g1, go1, load_compiled, reference_xml
+  from util import golden_xml
+
+  from mjlab_b200.asset_zoo import g1, go1, load_compiled
   from mjlab_b200.asset_zoo.scene import compile_scene
 
-  try:
-    g1_xml, go1_xml = reference_xml("g1"), reference_xml("go1")
-  except FileNotFoundError:
-    pytest.skip("reference checkout not present (GPU box)")
+  g1_xml, go1_xml = golden_xml("g1"), golden_xml("go1")
   sys.path.insert(0, str(__import__("pathlib").Path(__file__).resolve().parents[1] / "tools"))
   import compile_assets as ca
 

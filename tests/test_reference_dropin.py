@@ -1,6 +1,6 @@
 """The reference's own code on the B200 engine (VERDICT r01 item 2, SURVEY.md §7 step 3).
 
-``baseline/_ref`` holds the UNMODIFIED reference package (tools/install_reference.py); ``mjlab_b200.compat``
+``oracle/_ref`` holds the UNMODIFIED reference package (oracle/install_reference.py); ``mjlab_b200.compat``
 supplies ``mujoco_warp`` / ``warp`` / ``mujoco`` over libb2sim.so.  Executed from the reference's files:
 ``mjlab.sim.sim.Simulation`` + ``WarpBridge``/``TorchArray`` (sim/sim.py, sim/sim_data.py), ``expand_model_fields``
 (sim/randomization.py), ``Entity.initialize`` / ``_compute_indexing`` / ``EntityData`` (entity/entity.py,
@@ -20,7 +20,7 @@ import torch
 import refload
 from util import load_oracle, make_states, relerr
 
-pytestmark = [pytest.mark.skipif(not refload.available(), reason="baseline/_ref not installed")]
+pytestmark = [pytest.mark.skipif(not refload.available(), reason="oracle/_ref not installed")]
 
 N = 16
 

@@ -1,11 +1,11 @@
-"""The reference's OWN test files, unmodified and read where they lie (/root/reference/tests), executed against this
-repo's drop-in: ``mjlab`` is the unmodified package under baseline/_ref, ``mujoco`` / ``mujoco_warp`` / ``warp`` are
+"""The reference's OWN test files, unmodified (copied into oracle/_ref/tests by the build), executed against this
+repo's drop-in: ``mjlab`` is the unmodified package under oracle/_ref, ``mujoco`` / ``mujoco_warp`` / ``warp`` are
 mjlab_b200.compat, and the engine behind them is the product's CUDA source compiled for the host (tests/ref_runner.py).
 Only files whose subject is on the boundary of SURVEY.md §8(b) are run; the few cases that need what this image
 lacks are deselected by name, everything else must pass.
 With stand-ins for the absent RL / viewer wheels (tests/stubs, tests/ref_runner.py) the reference's task configs and
 ``ManagerBasedRlEnv`` import too: its smoke test passes and its hot loop is stepped on the engine (ref_env_cases.py).
-The GPU box has no /root/reference: the module is skipped there (and is not part of `-m gpu`)."""
+Where no reference checkout was found at build time there is no oracle/_ref and the module skips."""
 
 import re
 import subprocess
@@ -16,9 +16,9 @@ import pytest
 
 import refload
 
-REF_TESTS = Path("/root/reference/tests")
+REF_TESTS = refload.REF / "tests"
 pytestmark = pytest.mark.skipif(not (REF_TESTS.is_dir() and refload.available()),
-                                reason="needs /root/reference and baseline/_ref (build container only)")
+                                reason="oracle/_ref not installed (no reference checkout at build time)")
 
 CASES = [
   # file, deselect expression, minimum number of passing tests

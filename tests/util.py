@@ -2,7 +2,14 @@
 
 from __future__ import annotations
 
+from pathlib import Path
+
 import numpy as np
+
+
+def golden_xml(robot: str) -> str:
+  """MJCF text of a zoo robot (``g1``, ``go1``): the reference's asset_zoo file, stored as a fixture in tests/golden."""
+  return (Path(__file__).parent / "golden" / f"{robot}.xml").read_text()
 
 
 def _quat_mul(a, b):

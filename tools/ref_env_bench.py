@@ -1,5 +1,5 @@
 """Throughput of the REFERENCE's own env layer on this engine: ``ManagerBasedRlEnv.step`` (unmodified mjlab from
-baseline/_ref, its managers and task config) over libb2sim.so through mjlab_b200.compat - BASELINE's metric in the
+oracle/_ref, its managers and task config) over libb2sim.so through mjlab_b200.compat - BASELINE's metric in the
 reference's formulation of the caller, next to bench.py's fused MDP kernels.
 
   B2_REF_DEVICE=cuda:0 python tools/ref_env_bench.py [task=g1|go1|go1_rough] [num_envs=4096] [steps=50]
