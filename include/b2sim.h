@@ -84,9 +84,13 @@ const char* b2_field_name(b2_sim* sim, int which, int index);
 /* Tile a Model field to a real leading nworld dimension (reference randomization.py:20-55). */
 int b2_expand_model_field(b2_sim* sim, const char* name, void* cuda_stream, B2Tensor* out);
 
-/* Options: "iterations", "ls_iterations", "tolerance", "ls_tolerance", "ls_parallel",
- * "timestep", "integrator", "debug_outputs", "sorted_dispatch" (heavy-first launch order, default on), "fused_decimation" (b2_step_n as one launch; default off),
- * "dense_factor" (testing: always take the dense factorisation schedule instead of the dof-tree one). */
+/* Options (set and get): "iterations", "ls_iterations", "tolerance", "ls_tolerance", "timestep",
+ * "integrator", "solver" (1 CG, 2 Newton), "ls_parallel" (set only; accepted, the line search is exact),
+ * "sorted_dispatch" (heavy-first launch order, default on; set only), and the testing hooks
+ * "debug_outputs" (also write qfrc_bias, qfrc_smooth, qacc_smooth, qM, qfrc_constraint),
+ * "dense_factor" (always take the dense factorisation schedule instead of the dof-tree one) and
+ * "full_solver" (Newton on all dofs even when a leading block suffices).
+ * Read only: "smem_bytes_per_env", "maxcon", "reduced_block_cap". Any other key is an error. */
 int b2_set_option(b2_sim* sim, const char* key, double value);
 int b2_get_option(b2_sim* sim, const char* key, double* value);
 

@@ -939,12 +939,10 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
 #define FACTOR(sp) ldl_factor(H, invdiag, nv, SCHED, sp, lane)
 #define SOLVE(v, tree) ldl_solve(H, invdiag, v, nv, lane)
   // Phase-synchronous execution (dd.phase_sync): the kernel's code is ~200 KB against a 32 KB instruction cache,
-  // so the CTA's warps are re-aligned at every phase boundary and they fetch the same code together.
-  // Levels: 1 = major phases + one vote per Newton iteration, 2 = + the three segments of an iteration,
-  // 3 = + sub-phases of the smooth dynamics and the collision phase.
-  const int psync = dd.phase_sync;
-#define PSYNC_L(level) do { if (psync >= (level)) __syncthreads(); } while (0)
-#define PSYNC() PSYNC_L(1)
+  // so the CTA's warps are re-aligned at every phase boundary, at one vote per Newton iteration and between the
+  // three segments of an iteration, and they fetch the same code together.
+  const bool psync = dd.phase_sync != 0;
+#define PSYNC() do { if (psync) __syncthreads(); } while (0)
 #pragma unroll 1
   for (int i = threadIdx.x; i < m.ldl_nsparse; i += 32 * B2_WARPS_PER_CTA) s_sched[i] = m.ldl_sparse[i];
   if (threadIdx.x < 18) s_sched[m.ldl_nsparse + threadIdx.x] = (unsigned)m.ldl_start[threadIdx.x];
@@ -954,24 +952,11 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
   float* s = smem_all + (size_t)warp * L.total;
   const int nq = m.nq, nv = m.nv, nu = m.nu, nb = m.nbody, njnt = m.njnt;
   const int MC = L.maxcon, NLC = L.nlimcap;
-  uint32_t barphase = 0;
-  // Every warp is an independent worker.  With a ticket counter (dd.ticket) it pulls launch slots until the
-  // queue is empty - environments are handed out heavy-first (dd.world_order), so the warps of the whole grid
-  // finish together; without one it processes the single slot its position in the grid names.
-#pragma unroll 1
-  for (bool more = true; more;) {
-  int slot;
-  if (dd.ticket != nullptr) {
-    slot = 0;
-    if (lane == 0) slot = atomicAdd(dd.ticket, 1);
-    slot = __shfl_sync(FULL, slot, 0);
-  } else {
-    slot = blockIdx.x * B2_WARPS_PER_CTA + warp;
-    more = false;
-  }
-  if (slot >= dd.world_count) break;
+  // One warp per launch slot; environments are handed out heavy-first (dd.world_order).
+  const int slot = blockIdx.x * B2_WARPS_PER_CTA + warp;
+  if (slot >= dd.world_count) return;
   const int w = dd.world_order != nullptr ? dd.world_order[dd.world_base + slot] : dd.world_base + slot;
-  if (dd.world_mask != nullptr && dd.world_mask[w] == 0) continue;
+  if (dd.world_mask != nullptr && dd.world_mask[w] == 0) return;
 #ifdef B2_PHASE_TIMING
   long long tphase_ = clock64();
 #endif
@@ -984,7 +969,7 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
   const float* xfrc = dd.xfrc_applied.p + (size_t)w * dd.xfrc_applied.stride;
   {
     unsigned long long* bar = &bars[warp];
-    fence_async_smem();  // the previous environment's generic-proxy accesses precede this one's bulk writes
+    fence_async_smem();  // the barrier's initialisation precedes the bulk writes that complete on it
     __syncwarp();
     if (lane == 0) {
       uint32_t bytes = 4u * (dd.qpos.stride + dd.qvel.stride + dd.qacc_warmstart.stride);
@@ -994,8 +979,7 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
       bulk_g2s(qacc_ws, dd.qacc_warmstart.p + (size_t)w * dd.qacc_warmstart.stride, 4u * dd.qacc_warmstart.stride, bar);
     }
     __syncwarp();
-    mbar_wait(bar, barphase);
-    barphase ^= 1u;
+    mbar_wait(bar, 0);
   }
 
   PHASE_MARK(0);
@@ -1013,14 +997,9 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
   float* Mv = s + L.Mv; float* qfrc_c = s + L.qfrc_c;
   float* tmpv = s + L.tmpv; float* actf = s + L.actf;
 
-  // The decimation loop (manager_based_rl_env.py:109-114: ctrl held, `decimation` x sim.step) runs inside
-  // the launch: state vectors stay in shared memory between sub-steps.
-#pragma unroll 1
-  for (int sub = 0;; sub++) {
-  const bool lastsub = !STEP || sub + 1 >= dd.nsub;
   // Consumer-visible kinematics (poses, cvel, derived velocities) are observable only after the last sub-step
   // of a decimation loop: the launches before it skip those stores (and the poses of non-colliding geoms).
-  const bool emit = dd.emit != 0 && lastsub;
+  const bool emit = dd.emit != 0;
   bool ctrl_changed = false;
   // ---------------- phase 1: kinematics (lane per body, private walk down its ancestor chain) ----
   {
@@ -1402,7 +1381,6 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
     }
   }
   __syncwarp();
-  PSYNC_L(3);
   #pragma unroll 1
   for (int b = lane; b < nb; b += 32) {
     float a[6] = {0.f, 0.f, 0.f, -m.gravity[0], -m.gravity[1], -m.gravity[2]};
@@ -1435,7 +1413,6 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
   #pragma unroll 1
   for (int i = lane; i < nv; i += 32) tmpv[i] = 0.f;  // qfrc_actuator
   __syncwarp();
-  PSYNC_L(3);
   {
     const float* gp = MP(actuator_gainprm); const float* bp = MP(actuator_biasprm);
     const float* cr = MP(actuator_ctrlrange); const float* fr = MP(actuator_forcerange);
@@ -1449,7 +1426,7 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
       float g = gear[a];
       float len = qpos[m.jnt_qposadr[j]] * g, vel = qvel[m.jnt_dofadr[j]] * g;
       float c = ctrl[a];
-      if (STEP && (m.debug & 16)) { cdiff |= c != cprev[a]; cprev[a] = c; }
+      if (STEP) { cdiff |= c != cprev[a]; cprev[a] = c; }
       if (m.actuator_ctrllimited[a]) c = fminf(fmaxf(c, cr[2 * a]), cr[2 * a + 1]);
       float f = gp[10 * a] * c + bp[10 * a] + bp[10 * a + 1] * len + bp[10 * a + 2] * vel;
       if (m.actuator_forcelimited[a]) f = fminf(fmaxf(f, fr[2 * a]), fr[2 * a + 1]);
@@ -1460,7 +1437,6 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
     ctrl_changed = __any_sync(FULL, cdiff);
   }
   __syncwarp();
-  PSYNC_L(3);
   {
     const float* damp = MP(dof_damping); const float* stiff = MP(jnt_stiffness);
     const float* qpos0 = MP(qpos0);
@@ -1703,7 +1679,6 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
     PHASE_MARK(18);  // grid broadphase
     if (ncand > L.maxpair) { ncand = L.maxpair; overflow = 1; }
     __syncwarp();
-    PSYNC_L(3);
     const float* ggap = MP(geom_gap);
     const float* gfri = MP(geom_friction); const float* gsolref = MP(geom_solref);
     const float* gsolimp = MP(geom_solimp); const float* gsolmix = MP(geom_solmix);
@@ -2082,7 +2057,6 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
   // phase 7 left in H - on a reduced problem its leading block is the factor of the Schur complement).  The
   // Hessian scratch is unused, so its weight region holds the direction and the previous (grad, M^-1 grad).
   const bool cg = m.solver == SOL_CG_;
-  const bool ls_relstep = (m.debug & 8) != 0;
   float* search = cg ? gW : s + L.search;  // Newton: search = -grad in place
   float* cgM = gW + pad4i(nv); float* cgG0 = gW + 2 * pad4i(nv); float* cgM0 = gW + 3 * pad4i(nv);
   bool refine = false;  // active set unchanged: the Hessian factor of the previous iteration is still valid
@@ -2105,7 +2079,7 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
     // a_s,prev): the constraint part a - a_s of the previous solution is then the better guess (-0.95 Newton
     // iterations on those sub-steps; with an unchanged control the plain warm start is better by 0.4).  The
     // minimiser reached is the same; MuJoCo's rule (fall back to a_s when it is cheaper) still applies.
-    if ((m.debug & 16) && ctrl_changed) {
+    if (ctrl_changed) {
       const float* asp = dd.qacc_smooth_prev.p + (size_t)w * dd.qacc_smooth_prev.stride;
       #pragma unroll 1
       for (int i = lane; i < n; i += 32) qacc_ws[i] += qacc_smooth[i] - asp[i];
@@ -2248,7 +2222,8 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
         // (1e3..1e5 here) resolves improvements only down to ~1e-4, so "no measurable improvement" can still
         // leave a residual of several newtons in the constraint forces: the improvement test is honoured only
         // once the gradient is small against the forces it balances (|M a - f_smooth| vs |J^T f|).
-        const bool small = gn <= m.newton_small * fmaxf(fn, 1.f);
+        constexpr float newton_small = 1e-10f;
+        const bool small = gn <= newton_small * fmaxf(fn, 1.f);
         if (gradient < m.tolerance) { run = false; break; }
         // Exact termination: the cost is one quadratic per active set, and a Newton step with exact line
         // search lands on that quadratic's minimiser; if the active set did not change across the move, the
@@ -2264,7 +2239,7 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
       first = false;
     } while (0);
     PHASE_MARK(12);
-    PSYNC_L(2);
+    PSYNC();
     if (run && !refine && !cg) {
       // ---- Hessian H = M + J^T D_active J via per-body-pair 6x6 blocks -------------------------
       {  // leading block only: the rows of the eliminated dofs keep the factor of M (needed after the loop)
@@ -2337,7 +2312,7 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
       }
     }
     PHASE_MARK(13);
-    PSYNC_L(2);
+    PSYNC();
     if (run && !cg) {
       if (!refine) ldl_factor(H, invdiag, n, SCHED, treeok, lane, (nv - n) >> 2);
       #pragma unroll 1
@@ -2363,20 +2338,19 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
       __syncwarp();
     }
     PHASE_MARK(14);
-    PSYNC_L(2);
+    PSYNC();
     if (run) do {
       // ---- exact line search along `search` --------------------------------------------------
       symv(Mr, search, Mv, n, lane);
       MULJ(search, CJV0, LJV, false);
-      float g1 = 0.f, g2 = 0.f, sn = 0.f, gc = 0.f;
+      float g1 = 0.f, g2 = 0.f, sn = 0.f;
       #pragma unroll 1
       for (int i = lane; i < n; i += 32) {
         g1 += search[i] * (Ma[i] - qs[i]);
         g2 += 0.5f * search[i] * Mv[i];
         sn += search[i] * search[i];
-        gc += search[i] * qfrc_c[i];
       }
-      g1 = wsum(g1); g2 = wsum(g2); sn = sqrtf(wsum(sn)); gc = wsum(gc);
+      g1 = wsum(g1); g2 = wsum(g2); sn = sqrtf(wsum(sn));
       if (sn < MINVAL) { run = false; break; }
       float gtol = m.tolerance * m.ls_tolerance * sn / scale;
       // each lane keeps its rows in registers for the whole search (<= 2 contacts + 1 limit per lane)
@@ -2441,13 +2415,17 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
       };
       PHASE_MARK(15);
       float alpha = 0.f, d0, d1;
-      // slope at 0 = grad . search (grad = M a - f_smooth - J^T f, and J^T f is still in qfrc_c).  A Newton direction
-      // solves H search = -grad, so the curvature at 0 is -slope and the first trial step is 1: no evaluation at 0.
-      if (cg || (m.debug & 32)) ls_eval(0.f, d0, d1);
-      else { d0 = g1 - gc; d1 = -d0; }
+      // Slope and curvature at 0 are evaluated, for Newton and CG alike.  For a Newton direction (H search = -grad)
+      // they could be taken from grad . search with a first trial step of 1, one evaluation fewer per iteration;
+      // that saved no measurable time on the GPU, and the worst of 1024 stiff envs of the config-C parity states
+      // moved from 1.8e-4 to 3.3e-4.
+      ls_eval(0.f, d0, d1);
       if (d0 < 0.f) {
         float lo_a = 0.f, hi_a = -1.f;  // hi_a < 0: no upper bracket yet
-        const float dstop = fmaxf(gtol, m.ls_rtol * fabsf(d0));  // (ls_rtol: stop on a relative drop of the slope; 0 = exact)
+        // stop once the slope is 1e-3 of its value at 0 (emulated bench workload: 7.0 -> 3.4 evaluations per
+        // Newton iteration, iteration count unchanged: 4.665 -> 4.67)
+        constexpr float ls_rtol = 1e-3f;
+        const float dstop = fmaxf(gtol, ls_rtol * fabsf(d0));
         alpha = -d0 / d1;
         #pragma unroll 1
         for (int it = 0; it < m.ls_iterations; it++) {
@@ -2460,7 +2438,7 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
           // The derivative is piecewise linear: a Newton step taken inside the root's piece lands on the root, and
           // the next evaluation returns fp32 noise, never |d0| < gtol (gtol ~ 1e-8 |search|).  A step below a few
           // ulp of alpha is that situation: take it and stop instead of dithering until the bracket collapses.
-          if (ls_relstep && fabsf(nxt - alpha) <= 4e-7f * fabsf(alpha)) { alpha = nxt; break; }
+          if (fabsf(nxt - alpha) <= 4e-7f * fabsf(alpha)) { alpha = nxt; break; }
           alpha = nxt;
         }
       }
@@ -2501,7 +2479,7 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
     }
   }
 
-  if (STEP && (m.debug & 16)) {
+  if (STEP) {
     float* asp = dd.qacc_smooth_prev.p + (size_t)w * dd.qacc_smooth_prev.stride;
     #pragma unroll 1
     for (int i = lane; i < nv; i += 32) asp[i] = qacc_smooth[i];
@@ -2672,11 +2650,9 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
     }
     __syncwarp();
     if (lane == 0) dd.time.p[(size_t)w * dd.time.stride] += h;
-    if (lastsub) {
-      float* gws = dd.qacc_warmstart.p + (size_t)w * dd.qacc_warmstart.stride;
-      #pragma unroll 1
-      for (int i = lane; i < nv; i += 32) gws[i] = qacc[i];
-    }
+    float* gws = dd.qacc_warmstart.p + (size_t)w * dd.qacc_warmstart.stride;
+    #pragma unroll 1
+    for (int i = lane; i < nv; i += 32) gws[i] = qacc[i];
   }
   // outputs that live contiguously in shared memory leave through bulk (TMA) stores
   {
@@ -2690,7 +2666,7 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
     }
     fence_async_smem();
     __syncwarp();
-    if (lane == 0 && STEP && lastsub) {
+    if (lane == 0 && STEP) {
       bulk_s2g(gq, qpos, 4u * dd.qpos.stride);
       bulk_s2g(gv, qvel, 4u * dd.qvel.stride);
       bulk_commit_wait();
@@ -2706,11 +2682,4 @@ b2_step_kernel(const __grid_constant__ DevModel m, const __grid_constant__ DevDa
       dd.solver_cost.p[(size_t)w * dd.solver_cost.stride] = cost;
     }
   }
-  if (lastsub) break;
-  // next sub-step: qpos/qvel/ctrl/qfrc_applied are still in shared memory; warm start from this sub-step's solution
-  #pragma unroll 1
-  for (int i = lane; i < nv; i += 32) qacc_ws[i] = qacc[i];
-  __syncwarp();
-  }  // sub-step loop
-  }  // worker loop
 }

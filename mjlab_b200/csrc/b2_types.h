@@ -73,10 +73,9 @@ struct DevModel {
   int nq, nv, nu, nbody, njnt, ngeom, nsite, nsensor, nsensordata, npair, ncg, maxdepth;
   int ntri;  // nv*(nv+1)/2
   int maxcon, njmax;
-  int integrator, iterations, ls_iterations, debug, solver;
+  int integrator, iterations, ls_iterations, solver;
+  int debug;  // test hooks: 1 debug outputs, 2 dense LDL schedule, 4 Newton on all dofs
   float timestep, tolerance, ls_tolerance, impratio, meaninertia;
-  float newton_small;  // Newton: squared gradient norm relative to the squared force norm below which the improvement / unchanged-set stops apply (1e-10)
-  float ls_rtol;  // line search: stop when the slope has dropped to this fraction of its value at 0 (0: exact search)
   float gravity[3];
   // integer tables
   const int *body_parentid, *body_rootid, *body_jntadr, *body_jntnum, *body_dofadr, *body_dofnum;
@@ -136,7 +135,6 @@ struct DevModel {
 struct DevData {
   int nworld;
   int world_base, world_count;  // this launch covers launch slots [0, world_count) -> worlds from world_base
-  int nsub;  // sub-steps executed by one launch of the step kernel (decimation fused in-kernel)
   DArr qpos, qvel, ctrl, qacc_warmstart, qfrc_applied, xfrc_applied, act;
   DArr qacc, xpos, xquat, xmat, xipos, subtree_com, cvel, geom_xpos, geom_xmat, site_xpos,
       site_xmat, sensordata, actuator_force, time;
@@ -148,7 +146,6 @@ struct DevData {
   IArr ncon, nefc, solver_niter, contact_geom, overflow, solver_nd, solver_nls;
   int emit;                         // write consumer-visible kinematics (0 for all but the last sub-step of a decimation loop)
   int phase_sync;                   // CTA barriers at phase boundaries (every warp of the launch owns an environment)
-  int* ticket;                      // optional: work queue of launch slots (one atomic per environment)
   const int* world_order;           // optional: launch slot -> world (heavy-first dispatch)
   const unsigned char* world_mask;  // optional: worlds with mask 0 are skipped (masked forward)
 };

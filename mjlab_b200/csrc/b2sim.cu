@@ -50,6 +50,9 @@ struct Field {
   int64_t n = 0;         // elements per world
 };
 
+// b2_step_n runs this many environment partitions on internal streams once each holds at least 1024 environments
+static constexpr int B2_PARTITIONS = 2;
+
 struct b2_sim {
   int device = 0;
   int nworld = 0;
@@ -59,17 +62,11 @@ struct b2_sim {
   std::vector<void*> allocs;
   int64_t launches = 0;
   int* order = nullptr;       // heavy-first dispatch order (device)
-  int sorted_dispatch = 1;
-  int fused_decimation = 0;
-  int split_streams = 2;       // b2_step_n runs this many env partitions on internal streams
-  int reorder_every_substep = 1;  // heavy-first order recomputed before every sub-step (measured 447 vs 462 us: fresh Newton counts keep phase-synchronous CTAs balanced)
-  int phase_sync = 2;          // CTA barriers at phase boundaries, level 0..3 (instruction-cache locality; -14 % measured)
+  int sorted_dispatch = 1;     // heavy-first order, recomputed before every sub-step (measured 447 vs 462 us against once per
+                               // b2_step_n: fresh Newton counts keep phase-synchronous CTAs balanced)
   int has_convex = 0;          // the model has mesh / height-field collision pairs: kernels with the convex routines
-  int work_queue = 0;          // warps pull environments from a ticket counter (persistent grid)
-  int* tickets = nullptr;      // one counter per stream partition (device)
-  int resident_ctas = 0;       // co-resident CTAs of the step kernel on this device
-  cudaStream_t side[4] = {nullptr, nullptr, nullptr, nullptr};
-  cudaEvent_t ev_fork = nullptr, ev_join[4] = {nullptr, nullptr, nullptr, nullptr};  // measured slower (r01: 979 vs 733 us/sub-step): off by default
+  cudaStream_t side[B2_PARTITIONS] = {};  // b2_step_n: one internal stream per environment partition
+  cudaEvent_t ev_fork = nullptr, ev_join[B2_PARTITIONS] = {};
   size_t smem_bytes = 0;
   std::map<std::string, std::vector<double>> mf;  // host copy of float model arrays
   std::map<std::string, std::vector<int>> mi;
@@ -121,9 +118,8 @@ __device__ __forceinline__ int b2_order_key(int niter, int nd, int ncon, int nd_
 }
 __global__ void b2_order_kernel(const int* __restrict__ niter, int niter_stride, const int* __restrict__ ncon,
                                 int ncon_stride, const int* __restrict__ nd, int nd_stride, int nd_small,
-                                int base_world, int count, int* __restrict__ order, int* __restrict__ ticket) {
+                                int base_world, int count, int* __restrict__ order) {
   __shared__ int hist[128];
-  if (ticket != nullptr && threadIdx.x == 0) *ticket = 0;  // the step kernel's work queue starts empty
   __shared__ int base[128];
   for (int i = threadIdx.x; i < 128; i += blockDim.x) hist[i] = 0;
   __syncthreads();
@@ -241,33 +237,24 @@ static int add_idata(b2_sim* s, const char* name, IArr* arr, int n, int second =
   return 0;
 }
 
-static int launch(b2_sim* s, bool step, cudaStream_t st, int nsub = 1, int base = 0, int count = -1, int part = 0,
-                  int emit = 1, bool reorder = true) {
+static int launch(b2_sim* s, bool step, cudaStream_t st, int base = 0, int count = -1, int emit = 1) {
   if (count < 0) count = s->nworld;
-  s->hd.nsub = nsub;
   s->hd.emit = emit;
   s->hd.world_base = base;
   s->hd.world_count = count;
-  int grid = (count + B2_WARPS_PER_CTA - 1) / B2_WARPS_PER_CTA;
-  const bool queue = s->work_queue && s->tickets && s->resident_ctas > 0 && grid > s->resident_ctas;
-  int* ticket = queue ? s->tickets + part : nullptr;
+  const int grid = (count + B2_WARPS_PER_CTA - 1) / B2_WARPS_PER_CTA;
   if (step && s->sorted_dispatch && s->order && count >= 512 && s->hd.world_mask == nullptr) {
-    // (the order of the first sub-step of a decimation loop serves the whole loop: costs change little within it)
-    if (reorder || queue) {
-      b2_order_kernel<<<1, 1024, 0, st>>>(s->hd.solver_niter.p, s->hd.solver_niter.stride, s->hd.ncon.p,
-                                          s->hd.ncon.stride, s->hd.solver_nd.p, s->hd.solver_nd.stride,
-                                          s->hm.lay.ndcap, base, count, s->order, ticket);
-      s->launches++;
-    }
+    b2_order_kernel<<<1, 1024, 0, st>>>(s->hd.solver_niter.p, s->hd.solver_niter.stride, s->hd.ncon.p,
+                                        s->hd.ncon.stride, s->hd.solver_nd.p, s->hd.solver_nd.stride,
+                                        s->hm.lay.ndcap, base, count, s->order);
+    s->launches++;
     s->hd.world_order = s->order;
   } else {
     s->hd.world_order = nullptr;
-    if (queue) CUDA_OK(cudaMemsetAsync(ticket, 0, sizeof(int), st));
   }
-  s->hd.ticket = ticket;
-  // phase-synchronous warps need every warp of every CTA to own an environment (no early exits, no mask)
-  s->hd.phase_sync = (!queue && s->hd.world_mask == nullptr && count % B2_WARPS_PER_CTA == 0) ? s->phase_sync : 0;
-  if (queue) grid = s->resident_ctas;
+  // Phase-synchronous execution (CTA barriers at phase boundaries: instruction-cache locality, -14 % measured)
+  // needs every warp of every CTA to own an environment (no early exits, no mask).
+  s->hd.phase_sync = s->hd.world_mask == nullptr && count % B2_WARPS_PER_CTA == 0;
   if (step)
     if (s->has_convex) b2_step_kernel<3><<<grid, 32 * B2_WARPS_PER_CTA, s->smem_bytes, st>>>(s->hm, s->hd);
     else b2_step_kernel<1><<<grid, 32 * B2_WARPS_PER_CTA, s->smem_bytes, st>>>(s->hm, s->hd);
@@ -428,13 +415,7 @@ int b2_create(const B2ModelDesc* desc, int nworld, int ncon_per_world, int njmax
   if (m.nv > 64 || m.nbody > 64) { delete s; return fail("b2_create: nv and nbody must be <= 64"); }
   if (m.nv < 1) { delete s; return fail("b2_create: model has no degrees of freedom"); }
   m.integrator = geti("opt_integrator"); m.iterations = geti("opt_iterations");
-  m.ls_iterations = geti("opt_ls_iterations"); m.debug = 8 | 16 | 32;  // bit 3: relative-step stop of the line search; bit 4: shifted warm start after a control
-                         // change; bit 5: the line search evaluates its slope at 0 (off: grad . search and a first trial
-                         // step of 1 - one evaluation fewer per Newton iteration, no measurable time on the GPU, and
-                         // the worst of 1024 stiff envs of the config-C parity states moved from 1.8e-4 to 3.3e-4)
-  m.newton_small = 1e-10f;
-  m.ls_rtol = 1e-3f;  // line search stops once the slope is 1e-3 of its value at 0 (emulated bench workload: 7.0 -> 3.4
-                      // evaluations per Newton iteration, iteration count unchanged: 4.665 -> 4.67)
+  m.ls_iterations = geti("opt_ls_iterations");
   m.timestep = (float)getf("opt_timestep"); m.tolerance = (float)getf("opt_tolerance");
   m.ls_tolerance = (float)getf("opt_ls_tolerance"); m.impratio = (float)getf("opt_impratio");
   m.meaninertia = (float)getf("stat_meaninertia");
@@ -869,15 +850,7 @@ int b2_create(const B2ModelDesc* desc, int nworld, int ncon_per_world, int njmax
     if (cudaMalloc(&p, sizeof(int) * (size_t)nworld) != cudaSuccess) { b2_destroy(s); return fail("cudaMalloc(order)"); }
     s->allocs.push_back(p);
     s->order = (int*)p;
-    if (cudaMalloc(&p, sizeof(int) * 4) != cudaSuccess) { b2_destroy(s); return fail("cudaMalloc(tickets)"); }
-    s->allocs.push_back(p);
-    s->tickets = (int*)p;
-    cudaMemset(p, 0, sizeof(int) * 4);
-    int per_sm = 0, sms = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, b2_step_kernel<1>, 32 * B2_WARPS_PER_CTA, s->smem_bytes);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cuda_device);
-    s->resident_ctas = per_sm * sms;
-    for (int h = 0; h < 4; h++) {
+    for (int h = 0; h < B2_PARTITIONS; h++) {
       if (cudaStreamCreateWithFlags(&s->side[h], cudaStreamNonBlocking) != cudaSuccess ||
           cudaEventCreateWithFlags(&s->ev_join[h], cudaEventDisableTiming) != cudaSuccess) {
         b2_destroy(s);
@@ -921,7 +894,7 @@ int b2_destroy(b2_sim* s) {
   if (!s) return 0;
   DeviceGuard guard(s->device);
   for (void* p : s->allocs) cudaFree(p);
-  for (int h = 0; h < 4; h++) {
+  for (int h = 0; h < B2_PARTITIONS; h++) {
     if (s->side[h]) cudaStreamDestroy(s->side[h]);
     if (s->ev_join[h]) cudaEventDestroy(s->ev_join[h]);
   }
@@ -1001,17 +974,7 @@ int b2_set_option(b2_sim* s, const char* key, double v) {
   else if (k == "dense_factor") m.debug = (m.debug & ~2) | ((int)v ? 2 : 0);  // force the dense LDL schedule (tests)
   else if (k == "ls_parallel") { /* accepted for API parity; the line search here is exact */ }
   else if (k == "sorted_dispatch") s->sorted_dispatch = (int)v;
-  else if (k == "fused_decimation") s->fused_decimation = (int)v;
-  else if (k == "split_streams") s->split_streams = (int)v;
-  else if (k == "work_queue") s->work_queue = (int)v;
-  else if (k == "phase_sync") s->phase_sync = (int)v;
-  else if (k == "reorder_every_substep") s->reorder_every_substep = (int)v;
-  else if (k == "full_solver") m.debug = (m.debug & ~4) | ((int)v ? 4 : 0);  // Newton on all dofs even when a leading block suffices (tests, A/B)
-  else if (k == "warmstart_shift") m.debug = (m.debug & ~16) | ((int)v ? 16 : 0);  // previous solution moved by the change of qacc_smooth
-  else if (k == "ls_rtol") m.ls_rtol = (float)v;
-  else if (k == "ls_eval0") m.debug = (m.debug & ~32) | ((int)v ? 32 : 0);  // evaluate the line-search slope at 0 instead of using grad . search (A/B)
-  else if (k == "newton_small") m.newton_small = (float)v;
-  else if (k == "ls_relstep") m.debug = (m.debug & ~8) | ((int)v ? 8 : 0);  // line search stops on a relative step of a few ulp
+  else if (k == "full_solver") m.debug = (m.debug & ~4) | ((int)v ? 4 : 0);  // Newton on all dofs even when a leading block suffices (tests)
   else return fail("b2_set_option: unknown option '" + k + "'");
   return 0;
 }
@@ -1031,9 +994,6 @@ int b2_get_option(b2_sim* s, const char* key, double* v) {
   else if (k == "smem_bytes_per_env") *v = 4.0 * m.lay.total;
   else if (k == "maxcon") *v = m.maxcon;
   else if (k == "full_solver") *v = (m.debug >> 2) & 1;
-  else if (k == "work_queue") *v = s->work_queue;
-  else if (k == "phase_sync") *v = s->phase_sync;
-  else if (k == "resident_ctas") *v = s->resident_ctas;
   else if (k == "reduced_block_cap") *v = m.lay.ndcap;
   else return fail("b2_get_option: unknown option '" + k + "'");
   return 0;
@@ -1062,9 +1022,8 @@ int b2_step_n(b2_sim* s, int n, void* stream) {
   DeviceGuard guard(s->device);
   if (n <= 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
-  if (s->fused_decimation) return launch(s, true, st, n);
-  int np = std::min(std::max(s->split_streams, 1), 4);
-  if (np > 1 && n > 1 && s->nworld >= 1024 * np) {
+  const int np = B2_PARTITIONS;
+  if (n > 1 && s->nworld >= 1024 * np) {
     // Environments are independent, so the sub-steps of one partition need not wait for the others:
     // fork the partitions onto internal streams (event fork/join, CUDA-graph capturable). Each
     // partition keeps per-sub-step launches (phase-aligned warps, fresh heavy-first order) while
@@ -1076,14 +1035,14 @@ int b2_step_n(b2_sim* s, int n, void* stream) {
       if (count <= 0) break;
       CUDA_OK(cudaStreamWaitEvent(s->side[h], s->ev_fork, 0));
       for (int i = 0; i < n; i++)
-        if (launch(s, true, s->side[h], 1, base, count, h, i == n - 1, i == 0 || s->reorder_every_substep)) return 1;
+        if (launch(s, true, s->side[h], base, count, i == n - 1)) return 1;
       CUDA_OK(cudaEventRecord(s->ev_join[h], s->side[h]));
       CUDA_OK(cudaStreamWaitEvent(st, s->ev_join[h], 0));
     }
     return 0;
   }
   for (int i = 0; i < n; i++)
-    if (launch(s, true, st, 1, 0, -1, 0, i == n - 1, i == 0 || s->reorder_every_substep)) return 1;
+    if (launch(s, true, st, 0, -1, i == n - 1)) return 1;
   return 0;
 }
 

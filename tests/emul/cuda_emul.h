@@ -30,7 +30,6 @@ inline cudaError_t cudaMemcpy2DAsync(void* d, size_t dpitch, const void* s, size
   return 0;
 }
 inline cudaError_t cudaMemset(void* d, int v, size_t n) { memset(d, v, n); return 0; }
-inline cudaError_t cudaMemsetAsync(void* d, int v, size_t n, cudaStream_t = nullptr) { memset(d, v, n); return 0; }
 template <class S> inline cudaError_t cudaMemcpyToSymbol(S& sym, const void* s, size_t n) { memcpy(&sym, s, n); return 0; }
 template <class S> inline cudaError_t cudaMemcpyFromSymbol(void* d, const S& sym, size_t n) { memcpy(d, &sym, n); return 0; }
 inline cudaError_t cudaGetLastError() { return 0; }
@@ -47,10 +46,6 @@ inline cudaError_t cudaEventCreateWithFlags(cudaEvent_t* e, unsigned) { *e = (vo
 inline cudaError_t cudaEventDestroy(cudaEvent_t) { return 0; }
 inline cudaError_t cudaEventRecord(cudaEvent_t, cudaStream_t = nullptr) { return 0; }
 inline cudaError_t cudaStreamWaitEvent(cudaStream_t, cudaEvent_t, unsigned = 0) { return 0; }
-enum { cudaDevAttrMultiProcessorCount = 16 };
-// a "device" with two SMs holding one CTA each: a batch of more than two environments exercises the work queue
-template <class F> inline cudaError_t cudaOccupancyMaxActiveBlocksPerMultiprocessor(int* n, F, int, size_t) { *n = 1; return 0; }
-inline cudaError_t cudaDeviceGetAttribute(int* v, int, int) { *v = 2; return 0; }
 
 namespace cuda_emul {
 // run `kernel(args...)` for every CTA of the grid, one CTA at a time, on block.x fibers

@@ -194,10 +194,9 @@ def test_emulated_kernel_obstacle_course(lib):
   sim.close()
 
 
-def test_emulated_host_entry_fused_decimation_and_field_expansion(lib):
-  """Three host paths no CPU test could reach before: b2_step_host (host buffers in/out) equals b2_step_n, the
-  in-kernel decimation loop (`fused_decimation`) equals separate launches, and an expanded per-world model field
-  (geom_friction) is what the kernel reads."""
+def test_emulated_host_entry_and_field_expansion(lib):
+  """Two host paths no CPU test could reach before: b2_step_host (host buffers in/out) equals b2_step_n, and an
+  expanded per-world model field (geom_friction) is what the kernel reads."""
   from mjlab_b200.asset_zoo import load_compiled
 
   lib.b2_step_host.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
@@ -205,8 +204,8 @@ def test_emulated_host_entry_fused_decimation_and_field_expansion(lib):
   m = load_compiled("go1_flat")
   n, nq, nv, nu = 3, int(m.nq), int(m.nv), int(m.nu)
   st = make_states(m, n, seed=21)
-  ref, host, fused = EmulSim(lib, m, n), EmulSim(lib, m, n), EmulSim(lib, m, n)
-  for s in (ref, host, fused):
+  ref, host = EmulSim(lib, m, n), EmulSim(lib, m, n)
+  for s in (ref, host):
     s.load(st)
   ref.step(2)
   # host-buffer entry: ctrl from a dense host array, qpos/qvel back into dense host arrays
@@ -214,11 +213,6 @@ def test_emulated_host_entry_fused_decimation_and_field_expansion(lib):
   qpos_out, qvel_out = np.zeros((n, nq), dtype=np.float32), np.zeros((n, nv), dtype=np.float32)
   assert lib.b2_step_host(host.h, ctrl.ctypes.data, 2, qpos_out.ctypes.data, qvel_out.ctypes.data, None) == 0
   assert (qpos_out == ref.field("qpos")).all() and (qvel_out == ref.field("qvel")).all()
-  # decimation fused into one launch
-  lib.b2_set_option(fused.h, b"fused_decimation", 1.0)
-  fused.step(2)
-  assert np.abs(fused.field("qpos") - ref.field("qpos")).max() < 1e-6
-  assert np.abs(fused.field("qvel") - ref.field("qvel")).max() < 1e-5
   # per-world friction: world 0 keeps the model's value, the others get ice under their feet
   t = native.B2Tensor()
   assert lib.b2_expand_model_field(ref.h, b"geom_friction", None, ctypes.byref(t)) == 0
@@ -234,7 +228,7 @@ def test_emulated_host_entry_fused_decimation_and_field_expansion(lib):
   assert np.abs(qa[0] - qb[0]).max() == 0.0  # the untouched world: bit-identical
   # (only the feet have condim 3; a world whose contacts are all frictionless would not notice)
   assert max(np.abs(qa[w] - qb[w]).max() for w in range(1, n)) > 1e-3
-  for s in (ref, host, fused):
+  for s in (ref, host):
     s.close()
 
 
@@ -419,24 +413,22 @@ def test_emulated_kernel_synthetic_45dof_robot(lib):
   sim.close()
 
 
-def test_emulated_reduced_solver_and_work_queue(lib):
+def test_emulated_reduced_solver_matches_full_solver(lib):
   """The Newton solver on the constrained leading block (Schur complement of M onto the dofs any constraint
-  touches, the rest by back-substitution) gives the full-size solver's answer, and the ticket work queue
-  (persistent warps pulling environments) visits every environment exactly once."""
+  touches, the rest by back-substitution) gives the full-size solver's answer."""
   from mjlab_b200.asset_zoo import load_compiled
 
   m = load_compiled("g1_flat")
-  n = 5  # more environments than the emulated device holds CTAs (2): the queue hands out several per warp
+  n = 5
   sim = EmulSim(lib, m, n)
-  assert sim.option("reduced_block_cap") == 19 and sim.option("resident_ctas") == 2
+  assert sim.option("reduced_block_cap") == 19
   o = Oracle(m, nworld=n, maxcon=int(sim.option("maxcon")))
   st = make_states(m, n, seed=5)
   load_oracle(o, st)
   o.forward()
   res = {}
-  for mode, full, queue in (("reduced", 0, 0), ("full", 1, 0), ("queue", 0, 1)):
+  for mode, full in (("reduced", 0), ("full", 1)):
     lib.b2_set_option(sim.h, b"full_solver", float(full))
-    lib.b2_set_option(sim.h, b"work_queue", float(queue))
     sim.load(st)
     sim.field("qacc")[...] = 0
     sim.forward()
@@ -444,9 +436,8 @@ def test_emulated_reduced_solver_and_work_queue(lib):
     assert relerr(res[mode][0], o.qacc).max() < 1e-4, mode
     assert relerr(res[mode][1], o.qfrc_constraint).max() < 1e-4, mode
   assert (o.nefc.ravel() > 0).sum() >= 3
-  assert np.array_equal(res["reduced"][0], res["queue"][0])  # same arithmetic, different dispatch
   assert relerr(res["reduced"][0], res["full"][0]).max() < 1e-4
-  lib.b2_set_option(sim.h, b"work_queue", 1.0)
+  lib.b2_set_option(sim.h, b"full_solver", 0.0)
   load_oracle(o, st)
   sim.load(st)
   o.step()

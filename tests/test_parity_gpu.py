@@ -314,20 +314,21 @@ def test_masked_forward_only_touches_selected_worlds(g1_model):
   sim.close()
 
 
-def test_fused_decimation_matches_separate_steps(g1_model):
-  """b2_step_n(4) (one launch, state kept in shared memory) == 4 x b2_step, bit for bit."""
+def test_step_n_matches_separate_steps(g1_model):
+  """b2_step_n(4) == 4 x b2_step, bit for bit.  At 2048 worlds step_n runs two partitions on internal streams and
+  emits the consumer-visible kinematics on the last sub-step only."""
   from mjlab_b200.sim import Simulation, SimulationCfg
 
-  st = make_states(g1_model, 64, seed=17)
-  a = Simulation(64, SimulationCfg(), g1_model, "cuda:0")
-  b = Simulation(64, SimulationCfg(), g1_model, "cuda:0")
+  n = 2048
+  st = make_states(g1_model, n, seed=17)
+  a = Simulation(n, SimulationCfg(), g1_model, "cuda:0")
+  b = Simulation(n, SimulationCfg(), g1_model, "cuda:0")
   rng = np.random.default_rng(1)
-  xf = np.zeros((64, int(g1_model.nbody), 6), np.float32)
-  xf[:, 5] = rng.uniform(-10, 10, (64, 6))
+  xf = np.zeros((n, int(g1_model.nbody), 6), np.float32)
+  xf[:, 5] = rng.uniform(-10, 10, (n, 6))
   for s in (a, b):
     load_sim(s, st)
     s.data.xfrc_applied[:] = torch.tensor(xf, device="cuda:0")
-  b.set_option("fused_decimation", 1)
   for _ in range(4):
     a.step()
   b.step_n(4)
@@ -335,7 +336,6 @@ def test_fused_decimation_matches_separate_steps(g1_model):
   for f in ("qpos", "qvel", "qacc", "qacc_warmstart", "xpos", "sensordata", "contact_force"):
     assert (getattr(a.data, f)[:] == getattr(b.data, f)[:]).all(), f
   assert torch.allclose(a.data.time[:], b.data.time[:])
-  assert b.launch_count() < a.launch_count()
   a.close()
   b.close()
 

@@ -37,9 +37,7 @@ def timeit4(label, k=10):
   sim.data.qpos[:] = state[0]; sim.data.qvel[:] = state[1]; sim.data.qacc_warmstart[:] = state[2]
 if mode == "time":
   timeit("steady state (random actions)")
-  for k in (2, 3, 4, 1):
-    sim.set_option("split_streams", k); timeit4(f"step_n(4), {k} partition(s)/stream(s)")
-  sim.set_option("split_streams", 2)
+  timeit4("step_n(4)")
   sim.set_option("iterations", 1); timeit("iterations=1")
   sim.set_option("iterations", 0); timeit("iterations=0")
   sim.set_option("iterations", 10)

@@ -52,7 +52,7 @@ def main():
     ni = sim.data.solver_niter[:].float().mean().item()
     ov = int(sim.data.overflow[:].sum().item())
     print(f"{name}: n={a.n} {us:.1f} us/sub-step  {a.n / us:.2f} M env-substeps/s  ncon={nc:.1f} niter={ni:.2f} overflow={ov} "
-          f"smem/env={int(sim.get_option('smem_bytes_per_env'))} resident_ctas={int(sim.get_option('resident_ctas'))}")
+          f"smem/env={int(sim.get_option('smem_bytes_per_env'))}")
     sim.close()
 
 
