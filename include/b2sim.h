@@ -76,7 +76,9 @@ int b2_destroy(b2_sim* sim);
 /* Zero-copy view of a field. Pointers stay valid for the lifetime of the sim, except that
  * b2_expand_model_field re-points the named Model field.  The model-pointer table travels to the
  * kernels as a by-value launch parameter, so CUDA graphs captured before an expansion must be
- * re-captured (mjlab does: manager_based_rl_env.py:102-104; our Simulation does it lazily). */
+ * re-captured (mjlab does: manager_based_rl_env.py:102-104; our Simulation does it lazily).
+ * A Model view of body_pos, body_quat, jnt_pos, jnt_axis or qpos0 (from either call, at any nworld)
+ * turns off the kinematic records cached from them at create time, which also changes that table. */
 int b2_get_field(b2_sim* sim, int which, const char* name, B2Tensor* out);
 int b2_num_fields(b2_sim* sim, int which);
 const char* b2_field_name(b2_sim* sim, int which, int index);

@@ -178,6 +178,13 @@ static const ShapeSpec kModelShapes[] = {
     {"site_quat", 4}, {"actuator_gainprm", 10}, {"actuator_biasprm", 10},
     {"actuator_ctrlrange", 2}, {"actuator_forcerange", 2}, {"actuator_gear", 0}, {"qpos0", 0}};
 
+// Model arrays that the compact kinematic records (m.kinrec) copy at create time. Once a caller can write one of
+// them (an expanded per-world array, or a view of the shared one), the records may go stale: the kernel must then
+// read the arrays themselves (m.fastkin = 0).
+static bool in_kinrec(const std::string& name) {
+  return name == "body_pos" || name == "body_quat" || name == "jnt_pos" || name == "jnt_axis" || name == "qpos0";
+}
+
 static FArr* model_farr(DevModel& m, const std::string& name) {
 #define F_(x) if (name == #x) return &m.x;
   F_(body_pos) F_(body_quat) F_(body_ipos) F_(body_iquat) F_(body_mass) F_(body_subtreemass)
@@ -918,6 +925,7 @@ int b2_get_field(b2_sim* s, int which, const char* name, B2Tensor* out) {
   if (!s || !name || !out) return fail("b2_get_field: bad arguments");
   Field* f = find_field(s, which, name);
   if (!f) return fail(std::string("b2_get_field: unknown field '") + name + "'");
+  if (which != B2_DATA && in_kinrec(f->name)) s->hm.fastkin = 0;  // the caller may write the array
   fill_tensor(s, *f, out);
   return 0;
 }
@@ -935,6 +943,8 @@ int b2_expand_model_field(b2_sim* s, const char* name, void* stream, B2Tensor* o
   Field* f = find_field(s, B2_MODEL, name);
   if (!f || !f->farr) return fail(std::string("b2_expand_model_field: '") + name + "' is not an expandable model field");
   DeviceGuard guard(s->device);
+  // (also at one world, where nothing is tiled: the caller then writes the shared array itself)
+  if (in_kinrec(f->name)) s->hm.fastkin = 0;
   if (f->farr->stride == 0 && s->nworld > 1) {
     int n = f->farr->n;
     void* p = nullptr;
@@ -945,11 +955,6 @@ int b2_expand_model_field(b2_sim* s, const char* name, void* stream, B2Tensor* o
     s->launches++;
     CUDA_OK(cudaGetLastError());
     f->farr->p = (const float*)p; f->farr->stride = n;
-    {
-      std::string nm = name;
-      if (nm == "body_pos" || nm == "body_quat" || nm == "jnt_pos" || nm == "jnt_axis" || nm == "qpos0")
-        s->hm.fastkin = 0;  // the compact kinematic records mirror the shared arrays only
-    }
     f->ptr = p; f->stride[0] = n;
   }
   if (out) fill_tensor(s, *f, out);

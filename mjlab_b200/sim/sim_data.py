@@ -174,6 +174,10 @@ class EngineStruct:
     native.check(self._sim._lib.b2_get_field(self._sim._h, self._which, name.encode(), ctypes.byref(t)))
     tensor = tensor_from_b2(t, self._sim)
     self._tensors[name] = tensor
+    if self._which == 1:
+      # a writable model view can switch the engine off its cached kinematic records, which a captured graph holds
+      # by value: re-capture before the next replay
+      self._sim._graph_dirty = True
     return tensor
 
   def _drop(self, name: str) -> None:
