@@ -19,6 +19,20 @@ enum { OBJ_BODY = 1, OBJ_XBODY = 2, OBJ_GEOM = 5 };
 enum { INT_EULER = 0, INT_IMPLICITFAST = 3 };
 enum { SOL_PGS_ = 0, SOL_CG_ = 1, SOL_NEWTON_ = 2 };
 
+// The float model arrays a caller may expand per world, in DevModel's member order:
+// X(name, trailing width of the caller's view, element count in model sizes).  Width 1 is a 1-D view per world.
+#define B2_MODEL_FARRAYS(X)                                                                                       \
+  X(body_pos, 3, nbody) X(body_quat, 4, nbody) X(body_ipos, 3, nbody) X(body_iquat, 4, nbody)                    \
+  X(body_mass, 1, nbody) X(body_subtreemass, 1, nbody) X(body_inertia, 3, nbody) X(body_invweight0, 2, nbody)    \
+  X(jnt_pos, 3, njnt) X(jnt_axis, 3, njnt) X(jnt_range, 2, njnt) X(jnt_solref, 2, njnt) X(jnt_solimp, 5, njnt)   \
+  X(jnt_margin, 1, njnt) X(jnt_stiffness, 1, njnt)                                                               \
+  X(dof_armature, 1, nv) X(dof_damping, 1, nv) X(dof_frictionloss, 1, nv) X(dof_invweight0, 1, nv)               \
+  X(geom_size, 3, ngeom) X(geom_pos, 3, ngeom) X(geom_quat, 4, ngeom) X(geom_friction, 3, ngeom)                 \
+  X(geom_solref, 2, ngeom) X(geom_solimp, 5, ngeom) X(geom_solmix, 1, ngeom) X(geom_margin, 1, ngeom)            \
+  X(geom_gap, 1, ngeom) X(geom_rbound, 1, ngeom) X(geom_rgba, 4, ngeom) X(site_pos, 3, nsite)                    \
+  X(site_quat, 4, nsite) X(actuator_gainprm, 10, nu) X(actuator_biasprm, 10, nu) X(actuator_ctrlrange, 2, nu)    \
+  X(actuator_forcerange, 2, nu) X(actuator_gear, 1, nu) X(qpos0, 1, nq)
+
 // A float model array; `stride` is the per-world stride in floats (0 = shared by all worlds).
 struct FArr {
   const float* p;
@@ -123,12 +137,9 @@ struct DevModel {
   int ldl_start[18];
   int ldl_nsparse;
   // float arrays (expandable per world)
-  FArr body_pos, body_quat, body_ipos, body_iquat, body_mass, body_subtreemass, body_inertia,
-      body_invweight0, jnt_pos, jnt_axis, jnt_range, jnt_solref, jnt_solimp, jnt_margin,
-      jnt_stiffness, dof_armature, dof_damping, dof_frictionloss, dof_invweight0, geom_size,
-      geom_pos, geom_quat, geom_friction, geom_solref, geom_solimp, geom_solmix, geom_margin,
-      geom_gap, geom_rbound, geom_rgba, site_pos, site_quat, actuator_gainprm, actuator_biasprm,
-      actuator_ctrlrange, actuator_forcerange, actuator_gear, qpos0;
+#define B2_FARR_MEMBER(name, width, count) FArr name;
+  B2_MODEL_FARRAYS(B2_FARR_MEMBER)
+#undef B2_FARR_MEMBER
   Layout lay;
 };
 

@@ -4,8 +4,11 @@
 #include <string.h>
 
 #include <algorithm>
+#include <initializer_list>
 #include <map>
+#include <memory>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/b2sim.h"
@@ -68,8 +71,6 @@ struct b2_sim {
   cudaStream_t side[B2_PARTITIONS] = {};  // b2_step_n: one internal stream per environment partition
   cudaEvent_t ev_fork = nullptr, ev_join[B2_PARTITIONS] = {};
   size_t smem_bytes = 0;
-  std::map<std::string, std::vector<double>> mf;  // host copy of float model arrays
-  std::map<std::string, std::vector<int>> mi;
 };
 
 static int pad4(int n) { return (n + 3) & ~3; }
@@ -165,18 +166,66 @@ __global__ void b2_order_kernel(const int* __restrict__ niter, int niter_stride,
   }
 }
 
-// inner shapes of model float fields: dims after the (broadcast) world dimension
-struct ShapeSpec { const char* name; int second; };  // second = trailing dim (0 -> 1-D)
-static const ShapeSpec kModelShapes[] = {
-    {"body_pos", 3}, {"body_quat", 4}, {"body_ipos", 3}, {"body_iquat", 4}, {"body_mass", 0},
-    {"body_subtreemass", 0}, {"body_inertia", 3}, {"body_invweight0", 2}, {"jnt_pos", 3},
-    {"jnt_axis", 3}, {"jnt_range", 2}, {"jnt_solref", 2}, {"jnt_solimp", 5}, {"jnt_margin", 0},
-    {"jnt_stiffness", 0}, {"dof_armature", 0}, {"dof_damping", 0}, {"dof_frictionloss", 0},
-    {"dof_invweight0", 0}, {"geom_size", 3}, {"geom_pos", 3}, {"geom_quat", 4},
-    {"geom_friction", 3}, {"geom_solref", 2}, {"geom_solimp", 5}, {"geom_solmix", 0},
-    {"geom_margin", 0}, {"geom_gap", 0}, {"geom_rbound", 0}, {"geom_rgba", 4}, {"site_pos", 3},
-    {"site_quat", 4}, {"actuator_gainprm", 10}, {"actuator_biasprm", 10},
-    {"actuator_ctrlrange", 2}, {"actuator_forcerange", 2}, {"actuator_gear", 0}, {"qpos0", 0}};
+// Model sizes, as the descriptor's scalars give them.
+struct Sizes {
+  long long nq, nv, nu, nbody, njnt, ngeom, nsite, nsensor, npair, nstatic;
+};
+
+// The expandable float model arrays (b2_types.h: B2_MODEL_FARRAYS) with their view width and element count.
+struct FloatArray {
+  const char* name;
+  FArr DevModel::*member;
+  int width;
+  long long n;
+};
+static std::vector<FloatArray> float_arrays(const Sizes& z) {
+#define F_(name, width, count) {#name, &DevModel::name, width, width * z.count},
+  return {B2_MODEL_FARRAYS(F_)};
+#undef F_
+}
+
+// The integer model arrays the kernel reads.  Their values must satisfy lo <= v < hi (unchecked when lo == NO).
+// ALWAYS: required, with n elements; GRID: required like that when the model has a static grid (nstatic > 0);
+// OPTIONAL: asset and grid tables of any length, empty when absent.  The arrays callers can read as model fields
+// (`visible`) come first, in the order b2_field_name lists them.
+static constexpr long long NO = -(1ll << 40);
+enum Need { ALWAYS, GRID, OPTIONAL };
+struct IntArray {
+  const char* name;
+  const int* DevModel::*member;
+  long long n, lo, hi;
+  bool visible;
+  Need need;
+};
+static std::vector<IntArray> int_arrays(const Sizes& z) {
+#define I_(name, n, lo, hi, visible, need) {#name, &DevModel::name, n, lo, hi, visible, need}
+  return {
+      I_(geom_bodyid, z.ngeom, 0, z.nbody, true, ALWAYS), I_(site_bodyid, z.nsite, 0, z.nbody, true, ALWAYS),
+      I_(body_parentid, z.nbody, 0, z.nbody, true, ALWAYS), I_(body_rootid, z.nbody, 0, z.nbody, true, ALWAYS),
+      I_(jnt_type, z.njnt, 0, 4, true, ALWAYS), I_(jnt_qposadr, z.njnt, 0, z.nq, true, ALWAYS),
+      I_(jnt_dofadr, z.njnt, 0, z.nv, true, ALWAYS), I_(dof_bodyid, z.nv, 0, z.nbody, true, ALWAYS),
+      I_(geom_type, z.ngeom, 0, 9, true, ALWAYS), I_(geom_condim, z.ngeom, 1, 7, true, ALWAYS),
+      I_(geom_priority, z.ngeom, NO, -NO, true, ALWAYS), I_(actuator_trnid, z.nu, 0, z.njnt, true, ALWAYS),
+      I_(body_jntadr, z.nbody, -1, z.njnt, false, ALWAYS), I_(body_jntnum, z.nbody, 0, z.njnt + 1, false, ALWAYS),
+      I_(body_dofadr, z.nbody, -1, z.nv, false, ALWAYS), I_(body_dofnum, z.nbody, 0, z.nv + 1, false, ALWAYS),
+      I_(jnt_bodyid, z.njnt, 0, z.nbody, false, ALWAYS), I_(jnt_limited, z.njnt, 0, 2, false, ALWAYS),
+      I_(dof_jntid, z.nv, 0, z.njnt, false, ALWAYS), I_(dof_parentid, z.nv, -1, z.nv, false, ALWAYS),
+      I_(actuator_ctrllimited, z.nu, 0, 2, false, ALWAYS), I_(actuator_forcelimited, z.nu, 0, 2, false, ALWAYS),
+      I_(pair_geom1, z.npair, 0, z.ngeom, false, ALWAYS), I_(pair_geom2, z.npair, 0, z.ngeom, false, ALWAYS),
+      I_(sensor_objtype, z.nsensor, NO, -NO, false, ALWAYS), I_(sensor_objid, z.nsensor, NO, -NO, false, ALWAYS),
+      I_(sensor_reftype, z.nsensor, NO, -NO, false, ALWAYS), I_(sensor_refid, z.nsensor, NO, -NO, false, ALWAYS),
+      I_(sensor_intprm, 3 * z.nsensor, NO, -NO, false, ALWAYS), I_(sensor_adr, z.nsensor, 0, 1 << 20, false, ALWAYS),
+      I_(sensor_dim, z.nsensor, 0, 1 << 20, false, ALWAYS),
+      I_(geom_contype, z.ngeom, NO, -NO, false, GRID), I_(geom_conaffinity, z.ngeom, NO, -NO, false, GRID),
+      I_(static_geom, z.nstatic, 0, z.ngeom, false, GRID), I_(static_cell0, 2 * z.nstatic, 0, 1 << 20, false, GRID),
+      I_(dyn_cgeom, 0, 0, z.ngeom, false, OPTIONAL), I_(grid_start, 0, NO, -NO, false, OPTIONAL),
+      I_(grid_items, 0, 0, z.nstatic, false, OPTIONAL), I_(geom_dataid, 0, NO, -NO, false, OPTIONAL),
+      I_(mesh_vertadr, 0, NO, -NO, false, OPTIONAL), I_(mesh_vertnum, 0, NO, -NO, false, OPTIONAL),
+      I_(hfield_adr, 0, NO, -NO, false, OPTIONAL), I_(hfield_nrow, 0, NO, -NO, false, OPTIONAL),
+      I_(hfield_ncol, 0, NO, -NO, false, OPTIONAL),
+  };
+#undef I_
+}
 
 // Model arrays that the compact kinematic records (m.kinrec) copy at create time. Once a caller can write one of
 // them (an expanded per-world array, or a view of the shared one), the records may go stale: the kernel must then
@@ -185,64 +234,31 @@ static bool in_kinrec(const std::string& name) {
   return name == "body_pos" || name == "body_quat" || name == "jnt_pos" || name == "jnt_axis" || name == "qpos0";
 }
 
-static FArr* model_farr(DevModel& m, const std::string& name) {
-#define F_(x) if (name == #x) return &m.x;
-  F_(body_pos) F_(body_quat) F_(body_ipos) F_(body_iquat) F_(body_mass) F_(body_subtreemass)
-  F_(body_inertia) F_(body_invweight0) F_(jnt_pos) F_(jnt_axis) F_(jnt_range) F_(jnt_solref)
-  F_(jnt_solimp) F_(jnt_margin) F_(jnt_stiffness) F_(dof_armature) F_(dof_damping)
-  F_(dof_frictionloss) F_(dof_invweight0) F_(geom_size) F_(geom_pos) F_(geom_quat)
-  F_(geom_friction) F_(geom_solref) F_(geom_solimp) F_(geom_solmix) F_(geom_margin) F_(geom_gap)
-  F_(geom_rbound) F_(geom_rgba) F_(site_pos) F_(site_quat) F_(actuator_gainprm)
-  F_(actuator_biasprm) F_(actuator_ctrlrange) F_(actuator_forcerange) F_(actuator_gear) F_(qpos0)
-#undef F_
-  return nullptr;
+// A zeroed per-world Data array (DArr or IArr) whose caller-visible view is (nworld, *inner): rows padded to 16 B.
+template <class Arr>
+static int add_data(b2_sim* s, const char* name, Arr* arr, std::initializer_list<int> inner) {
+  using T = std::remove_pointer_t<decltype(arr->p)>;
+  Field f;
+  f.name = name; f.dtype = std::is_same<T, int>::value ? B2_I32 : B2_F32;
+  f.ndim = 1 + (int)inner.size();
+  f.n = 1;
+  for (int k : inner) f.n *= k;
+  const int stride = pad4(std::max((int)f.n, 1));
+  f.shape[0] = s->nworld; f.stride[0] = stride;
+  for (int k = f.ndim - 1; k >= 1; k--) {
+    f.shape[k] = inner.begin()[k - 1];
+    f.stride[k] = k == f.ndim - 1 ? 1 : f.stride[k + 1] * f.shape[k + 1];
+  }
+  size_t bytes = sizeof(T) * (size_t)s->nworld * stride;
+  CUDA_OK(cudaMalloc(&f.ptr, bytes));
+  s->allocs.push_back(f.ptr);
+  CUDA_OK(cudaMemset(f.ptr, 0, bytes));
+  arr->p = (T*)f.ptr; arr->stride = stride; arr->n = (int)f.n;
+  s->data_fields.push_back(f);
+  return 0;
 }
 
-static int add_data(b2_sim* s, const char* name, DArr* arr, int n, int second = 0) {
-  int stride = pad4(std::max(n, 0));
-  if (stride == 0) stride = 4;
-  void* p = nullptr;
-  size_t bytes = sizeof(float) * (size_t)s->nworld * stride;
-  CUDA_OK(cudaMalloc(&p, bytes));
-  CUDA_OK(cudaMemset(p, 0, bytes));
-  s->allocs.push_back(p);
-  arr->p = (float*)p; arr->stride = stride; arr->n = n;
-  Field f;
-  f.name = name; f.ptr = p; f.dtype = B2_F32; f.n = n;
-  if (second == 9) {  // rotation matrices are exposed as (nworld, n, 3, 3) like mjwarp's mat33 arrays
-    f.ndim = 4; f.shape[0] = s->nworld; f.shape[1] = n / 9; f.shape[2] = 3; f.shape[3] = 3;
-    f.stride[0] = stride; f.stride[1] = 9; f.stride[2] = 3; f.stride[3] = 1;
-  } else if (second > 0) {
-    f.ndim = 3; f.shape[0] = s->nworld; f.shape[1] = n / second; f.shape[2] = second;
-    f.stride[0] = stride; f.stride[1] = second; f.stride[2] = 1;
-  } else {
-    f.ndim = 2; f.shape[0] = s->nworld; f.shape[1] = n;
-    f.stride[0] = stride; f.stride[1] = 1;
-  }
-  s->data_fields.push_back(f);
-  return 0;
-}
-static int add_idata(b2_sim* s, const char* name, IArr* arr, int n, int second = 0) {
-  int stride = pad4(std::max(n, 1));
-  void* p = nullptr;
-  size_t bytes = sizeof(int) * (size_t)s->nworld * stride;
-  CUDA_OK(cudaMalloc(&p, bytes));
-  CUDA_OK(cudaMemset(p, 0, bytes));
-  s->allocs.push_back(p);
-  arr->p = (int*)p; arr->stride = stride; arr->n = n;
-  Field f;
-  f.name = name; f.ptr = p; f.dtype = B2_I32; f.n = n;
-  if (second > 0) {
-    f.ndim = 3; f.shape[0] = s->nworld; f.shape[1] = n / second; f.shape[2] = second;
-    f.stride[0] = stride; f.stride[1] = second; f.stride[2] = 1;
-  } else if (n == 1) {
-    f.ndim = 1; f.shape[0] = s->nworld; f.stride[0] = stride;
-  } else {
-    f.ndim = 2; f.shape[0] = s->nworld; f.shape[1] = n; f.stride[0] = stride; f.stride[1] = 1;
-  }
-  s->data_fields.push_back(f);
-  return 0;
-}
+static std::vector<float> to_float(const std::vector<double>& v) { return std::vector<float>(v.begin(), v.end()); }
 
 static int launch(b2_sim* s, bool step, cudaStream_t st, int base = 0, int count = -1, int emit = 1) {
   if (count < 0) count = s->nworld;
@@ -292,8 +308,8 @@ int b2_phase_cycles(unsigned long long* out32) {
 #endif
 }
 
-// Sizes and index ranges of the model table (mjModel field names).  Returns "" when consistent.
-static std::string validate_desc(const B2ModelDesc* desc) {
+// Sizes, dtypes and index ranges of the model table (mjModel field names).  Returns "" when consistent.
+static std::string validate_desc(const B2ModelDesc* desc, Sizes* out) {
   std::map<std::string, const B2Array*> by;
   for (int i = 0; i < desc->narray; i++) {
     const B2Array& a = desc->arrays[i];
@@ -307,142 +323,125 @@ static std::string validate_desc(const B2ModelDesc* desc) {
     *out = it->second->dtype == B2_I32 ? ((const int32_t*)it->second->data)[0] : (long long)((const double*)it->second->data)[0];
     return true;
   };
-  long long nq, nv, nu, nbody, njnt, ngeom, nsite, nsensor, npair, nstatic = 0;
-  if (!scalar("nq", &nq) || !scalar("nv", &nv) || !scalar("nu", &nu) || !scalar("nbody", &nbody) || !scalar("njnt", &njnt) ||
-      !scalar("ngeom", &ngeom) || !scalar("nsite", &nsite) || !scalar("nsensor", &nsensor) || !scalar("npair", &npair))
+  Sizes z;
+  z.nstatic = 0;
+  if (!scalar("nq", &z.nq) || !scalar("nv", &z.nv) || !scalar("nu", &z.nu) || !scalar("nbody", &z.nbody) ||
+      !scalar("njnt", &z.njnt) || !scalar("ngeom", &z.ngeom) || !scalar("nsite", &z.nsite) ||
+      !scalar("nsensor", &z.nsensor) || !scalar("npair", &z.npair))
     return "missing size scalar (nq nv nu nbody njnt ngeom nsite nsensor npair)";
-  scalar("nstatic", &nstatic);
-  if (nq < 1 || nv < 1 || nbody < 1 || nu < 0 || njnt < 0 || ngeom < 0 || nsite < 0 || nsensor < 0 || npair < 0 || nstatic < 0)
+  scalar("nstatic", &z.nstatic);
+  if (z.nq < 1 || z.nv < 1 || z.nbody < 1 || z.nu < 0 || z.njnt < 0 || z.ngeom < 0 || z.nsite < 0 || z.nsensor < 0 ||
+      z.npair < 0 || z.nstatic < 0)
     return "negative or zero model size";
-  struct Req { const char* name; int dtype; long long n; long long lo, hi; };  // index range checked for lo <= v < hi
-  const long long NO = -(1ll << 40);
-  std::vector<Req> req = {
-    {"body_parentid", B2_I32, nbody, 0, nbody}, {"body_rootid", B2_I32, nbody, 0, nbody}, {"body_jntadr", B2_I32, nbody, -1, njnt},
-    {"body_jntnum", B2_I32, nbody, 0, njnt + 1}, {"body_dofadr", B2_I32, nbody, -1, nv}, {"body_dofnum", B2_I32, nbody, 0, nv + 1},
-    {"jnt_type", B2_I32, njnt, 0, 4}, {"jnt_qposadr", B2_I32, njnt, 0, nq}, {"jnt_dofadr", B2_I32, njnt, 0, nv},
-    {"jnt_bodyid", B2_I32, njnt, 0, nbody}, {"jnt_limited", B2_I32, njnt, 0, 2}, {"dof_bodyid", B2_I32, nv, 0, nbody},
-    {"dof_jntid", B2_I32, nv, 0, njnt}, {"dof_parentid", B2_I32, nv, -1, nv}, {"geom_type", B2_I32, ngeom, 0, 9},
-    {"geom_bodyid", B2_I32, ngeom, 0, nbody}, {"geom_condim", B2_I32, ngeom, 1, 7}, {"geom_priority", B2_I32, ngeom, NO, -NO},
-    {"site_bodyid", B2_I32, nsite, 0, nbody}, {"actuator_trnid", B2_I32, nu, 0, njnt},
-    {"actuator_ctrllimited", B2_I32, nu, 0, 2}, {"actuator_forcelimited", B2_I32, nu, 0, 2},
-    {"pair_geom1", B2_I32, npair, 0, ngeom}, {"pair_geom2", B2_I32, npair, 0, ngeom},
-    {"sensor_objtype", B2_I32, nsensor, NO, -NO}, {"sensor_objid", B2_I32, nsensor, NO, -NO}, {"sensor_reftype", B2_I32, nsensor, NO, -NO},
-    {"sensor_refid", B2_I32, nsensor, NO, -NO}, {"sensor_intprm", B2_I32, 3 * nsensor, NO, -NO}, {"sensor_adr", B2_I32, nsensor, 0, 1 << 20},
-    {"sensor_dim", B2_I32, nsensor, 0, 1 << 20},
-    {"body_pos", B2_F64, 3 * nbody}, {"body_quat", B2_F64, 4 * nbody}, {"body_ipos", B2_F64, 3 * nbody}, {"body_iquat", B2_F64, 4 * nbody},
-    {"body_mass", B2_F64, nbody}, {"body_subtreemass", B2_F64, nbody}, {"body_inertia", B2_F64, 3 * nbody}, {"body_invweight0", B2_F64, 2 * nbody},
-    {"jnt_pos", B2_F64, 3 * njnt}, {"jnt_axis", B2_F64, 3 * njnt}, {"jnt_range", B2_F64, 2 * njnt}, {"jnt_solref", B2_F64, 2 * njnt},
-    {"jnt_solimp", B2_F64, 5 * njnt}, {"jnt_margin", B2_F64, njnt}, {"jnt_stiffness", B2_F64, njnt}, {"dof_armature", B2_F64, nv},
-    {"dof_damping", B2_F64, nv}, {"dof_frictionloss", B2_F64, nv}, {"dof_invweight0", B2_F64, nv}, {"geom_size", B2_F64, 3 * ngeom},
-    {"geom_pos", B2_F64, 3 * ngeom}, {"geom_quat", B2_F64, 4 * ngeom}, {"geom_friction", B2_F64, 3 * ngeom}, {"geom_solref", B2_F64, 2 * ngeom},
-    {"geom_solimp", B2_F64, 5 * ngeom}, {"geom_solmix", B2_F64, ngeom}, {"geom_margin", B2_F64, ngeom}, {"geom_gap", B2_F64, ngeom},
-    {"geom_rbound", B2_F64, ngeom}, {"geom_rgba", B2_F64, 4 * ngeom}, {"site_pos", B2_F64, 3 * nsite}, {"site_quat", B2_F64, 4 * nsite},
-    {"actuator_gainprm", B2_F64, 10 * nu}, {"actuator_biasprm", B2_F64, 10 * nu}, {"actuator_ctrlrange", B2_F64, 2 * nu},
-    {"actuator_forcerange", B2_F64, 2 * nu}, {"actuator_gear", B2_F64, nu}, {"qpos0", B2_F64, nq},
-  };
-  if (nstatic > 0) {
-    req.push_back({"geom_contype", B2_I32, ngeom, NO, -NO});
-    req.push_back({"geom_conaffinity", B2_I32, ngeom, NO, -NO});
-    req.push_back({"static_geom", B2_I32, nstatic, 0, ngeom});
-    req.push_back({"static_cell0", B2_I32, 2 * nstatic, 0, 1 << 20});
-    req.push_back({"grid_params", B2_F64, 5});
-  }
-  for (const Req& r : req) {
-    auto it = by.find(r.name);
+  // the element count (of a required array), the dtype and the index range of one array
+  auto check = [&](const char* name, int dtype, bool required, long long n, long long lo, long long hi) -> std::string {
+    auto it = by.find(name);
     long long have = it == by.end() ? 0 : it->second->n;
-    if (have != r.n) return std::string("array '") + r.name + "' has " + std::to_string(have) + " elements, expected " + std::to_string(r.n);
-    if (r.n == 0) continue;
-    if (it->second->dtype != r.dtype) return std::string("array '") + r.name + "' has the wrong dtype";
-    if (r.dtype == B2_I32 && r.lo != NO) {
+    if (required && have != n)
+      return std::string("array '") + name + "' has " + std::to_string(have) + " elements, expected " + std::to_string(n);
+    if (have == 0) return "";
+    if (it->second->dtype != dtype) return std::string("array '") + name + "' has the wrong dtype";
+    if (lo != NO) {
       const int32_t* v = (const int32_t*)it->second->data;
-      for (long long i = 0; i < r.n; i++)
-        if (v[i] < r.lo || v[i] >= r.hi) return std::string("array '") + r.name + "' holds an index out of range";
+      for (long long i = 0; i < have; i++)
+        if (v[i] < lo || v[i] >= hi) return std::string("array '") + name + "' holds an index out of range";
     }
+    return "";
+  };
+  std::string why;
+  for (const IntArray& a : int_arrays(z)) {
+    bool required = a.need == ALWAYS || (a.need == GRID && z.nstatic > 0);
+    if (!(why = check(a.name, B2_I32, required, a.n, a.lo, a.hi)).empty()) return why;
   }
-  for (const char* k : {"dyn_cgeom", "grid_items"}) {
-    auto it = by.find(k);
-    if (it == by.end()) continue;
-    if (it->second->dtype != B2_I32) return std::string("array '") + k + "' has the wrong dtype";
-    long long hi = std::string(k) == "dyn_cgeom" ? ngeom : nstatic;
-    const int32_t* v = (const int32_t*)it->second->data;
-    for (long long i = 0; i < it->second->n; i++)
-      if (v[i] < 0 || v[i] >= hi) return std::string("array '") + k + "' holds an index out of range";
-  }
+  for (const FloatArray& a : float_arrays(z))
+    if (!(why = check(a.name, B2_F64, true, a.n, NO, -NO)).empty()) return why;
+  if (z.nstatic > 0 && !(why = check("grid_params", B2_F64, true, 5, NO, -NO)).empty()) return why;
   {  // parents precede children (the kinematic walks and the factorisation schedule rely on it)
-    const int32_t* bp = (const int32_t*)by["body_parentid"]->data;
-    for (long long b = 1; b < nbody; b++) if (bp[b] >= b) return "body_parentid: parents must precede children";
-    const int32_t* dp = (const int32_t*)by["dof_parentid"]->data;
-    for (long long d = 0; d < nv; d++) if (dp[d] >= d) return "dof_parentid: parents must precede children";
+    const int32_t* bp = (const int32_t*)by.at("body_parentid")->data;
+    for (long long b = 1; b < z.nbody; b++) if (bp[b] >= b) return "body_parentid: parents must precede children";
+    const int32_t* dp = (const int32_t*)by.at("dof_parentid")->data;
+    for (long long d = 0; d < z.nv; d++) if (dp[d] >= d) return "dof_parentid: parents must precede children";
   }
+  *out = z;
   return "";
 }
 
-int b2_create(const B2ModelDesc* desc, int nworld, int ncon_per_world, int njmax, int cuda_device,
-              b2_sim** out) {
-  if (!desc || !out || nworld <= 0) return fail("b2_create: bad arguments");
+// What b2_create derives from the descriptor on the host: the model's sizes, options and shared-memory layout (m,
+// whose pointers setup_device sets) and every table that setup_device uploads.
+struct HostModel {
+  Sizes z;
+  DevModel m;
+  int has_convex = 0;
+  size_t smem_bytes = 0;
+  std::map<std::string, std::vector<int>> mi;  // the descriptor's arrays
+  std::map<std::string, std::vector<double>> mf;
+  std::vector<int> depth, chain, cslot, cgeom, fixed_geom, posegeom;
+  std::vector<unsigned long long> dofmask, ancmask, submask, dofbody;
+  std::vector<float> kinrec, fixed_pose, static_pose;
+  std::vector<unsigned> pair_word, ldl_dense, ldl_sparse;
+  std::vector<int> hf_geom, hf_slot, hf_start, hf_pairs, hfd, nh;  // height-field pairs grouped by field (m.nhf > 0)
+  std::vector<float> hf_box;
+  // A descriptor array by name.  After validate_desc only optional arrays can be absent: they read as empty.
+  const std::vector<int>& ints(const std::string& k) const {
+    static const std::vector<int> none;
+    auto it = mi.find(k);
+    return it == mi.end() ? none : it->second;
+  }
+  const std::vector<double>& floats(const std::string& k) const {
+    static const std::vector<double> none;
+    auto it = mf.find(k);
+    return it == mf.end() ? none : it->second;
+  }
+  double scalar(const char* k) const {  // 0 when absent
+    if (!ints(k).empty()) return ints(k)[0];
+    return floats(k).empty() ? 0.0 : floats(k)[0];
+  }
+};
+
+// The host stage of b2_create: every check that can reject the descriptor, and every derived table.  No CUDA call.
+static int plan_model(const B2ModelDesc* desc, int ncon_per_world, int njmax, HostModel& h) {
   {
-    std::string why = validate_desc(desc);  // host-only: a malformed table must not reach the index loops
+    std::string why = validate_desc(desc, &h.z);  // a malformed table must not reach the index loops
     if (!why.empty()) return fail("b2_create: " + why);
   }
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-    return fail("b2_create: no CUDA device available (this library has no CPU path)");
-  if (cuda_device < 0 || cuda_device >= ndev) return fail("b2_create: bad cuda_device");
-  DeviceGuard guard(cuda_device);
-  b2_sim* s = new b2_sim();
-  s->device = cuda_device;
-  s->nworld = nworld;
   for (int i = 0; i < desc->narray; i++) {
     const B2Array& a = desc->arrays[i];
-    if (a.dtype == B2_I32) {
-      s->mi[a.name] = std::vector<int>((const int32_t*)a.data, (const int32_t*)a.data + a.n);
-    } else if (a.dtype == B2_F64) {
-      s->mf[a.name] = std::vector<double>((const double*)a.data, (const double*)a.data + a.n);
-    } else {
-      delete s;
-      return fail("b2_create: unsupported array dtype");
-    }
+    if (a.dtype == B2_I32) h.mi[a.name].assign((const int32_t*)a.data, (const int32_t*)a.data + a.n);
+    else h.mf[a.name].assign((const double*)a.data, (const double*)a.data + a.n);
   }
-  auto geti = [&](const char* k) -> int {
-    if (s->mi.count(k)) return s->mi[k].empty() ? 0 : s->mi[k][0];
-    if (s->mf.count(k)) return (int)s->mf[k][0];
-    return 0;
-  };
-  auto getf = [&](const char* k) -> double {
-    if (s->mf.count(k)) return s->mf[k][0];
-    if (s->mi.count(k)) return s->mi[k][0];
-    return 0.0;
-  };
-  DevModel& m = s->hm;
+  auto geti = [&](const char* k) { return (int)h.scalar(k); };
+  DevModel& m = h.m;
   memset(&m, 0, sizeof(m));
   m.nq = geti("nq"); m.nv = geti("nv"); m.nu = geti("nu"); m.nbody = geti("nbody");
   m.njnt = geti("njnt"); m.ngeom = geti("ngeom"); m.nsite = geti("nsite");
   m.nsensor = geti("nsensor"); m.nsensordata = geti("nsensordata"); m.npair = geti("npair");
   m.ntri = m.nv * (m.nv + 1) / 2;
-  if (m.nv > 64 || m.nbody > 64) { delete s; return fail("b2_create: nv and nbody must be <= 64"); }
-  if (m.nv < 1) { delete s; return fail("b2_create: model has no degrees of freedom"); }
+  if (m.nv > 64 || m.nbody > 64) return fail("b2_create: nv and nbody must be <= 64");
   m.integrator = geti("opt_integrator"); m.iterations = geti("opt_iterations");
   m.ls_iterations = geti("opt_ls_iterations");
-  m.timestep = (float)getf("opt_timestep"); m.tolerance = (float)getf("opt_tolerance");
-  m.ls_tolerance = (float)getf("opt_ls_tolerance"); m.impratio = (float)getf("opt_impratio");
-  m.meaninertia = (float)getf("stat_meaninertia");
+  m.timestep = (float)h.scalar("opt_timestep"); m.tolerance = (float)h.scalar("opt_tolerance");
+  m.ls_tolerance = (float)h.scalar("opt_ls_tolerance"); m.impratio = (float)h.scalar("opt_impratio");
+  m.meaninertia = (float)h.scalar("stat_meaninertia");
   for (int k = 0; k < 3; k++) m.gravity[k] = (float)desc->gravity[k];
-  if (geti("opt_cone") != 0) { delete s; return fail("b2_create: only pyramidal cones are supported"); }
+  if (geti("opt_cone") != 0) return fail("b2_create: only pyramidal cones are supported");
   m.solver = geti("opt_solver");
-  if (m.solver != SOL_NEWTON_ && m.solver != SOL_CG_) {
-    delete s;
+  if (m.solver != SOL_NEWTON_ && m.solver != SOL_CG_)
     return fail("b2_create: solver must be Newton or CG (PGS works on the dual problem and is not implemented)");
-  }
   m.maxcon = ncon_per_world > 0 ? std::min(ncon_per_world, 255) : 48;
   m.njmax = njmax > 0 ? njmax : 300;
 
   // ---- derived integer tables ---------------------------------------------------------------
-  const std::vector<int>& parent = s->mi["body_parentid"];
-  const std::vector<int>& dofadr = s->mi["body_dofadr"];
-  const std::vector<int>& dofnum = s->mi["body_dofnum"];
+  const std::vector<int>& parent = h.ints("body_parentid");
+  const std::vector<int>& dofadr = h.ints("body_dofadr");
+  const std::vector<int>& dofnum = h.ints("body_dofnum");
+  const std::vector<int>& geom_bodyid = h.ints("geom_bodyid");
+  const std::vector<int>& gt = h.ints("geom_type");
+  const std::vector<int>& pg1 = h.ints("pair_geom1");
+  const std::vector<int>& pg2 = h.ints("pair_geom2");
   int nb = m.nbody;
-  std::vector<int> depth(nb, 0);
-  std::vector<unsigned long long> dofmask(nb, 0ull), ancmask(nb, 0ull);
+  std::vector<int>& depth = h.depth;
+  std::vector<unsigned long long> &dofmask = h.dofmask, &ancmask = h.ancmask;
+  depth.assign(nb, 0); dofmask.assign(nb, 0ull); ancmask.assign(nb, 0ull);
   int maxdepth = 1;
   ancmask[0] = 1ull;
   for (int b = 1; b < nb; b++) {
@@ -452,35 +451,35 @@ int b2_create(const B2ModelDesc* desc, int nworld, int ncon_per_world, int njmax
     for (int k = 0; k < dofnum[b]; k++) dofmask[b] |= 1ull << (dofadr[b] + k);
     ancmask[b] = ancmask[parent[b]] | (1ull << b);
   }
-  std::vector<int> chain((size_t)nb * maxdepth, 0);
+  h.chain.assign((size_t)nb * maxdepth, 0);
   for (int b = 1; b < nb; b++) {
     int c = b;
-    for (int k = depth[b] - 1; k >= 0; k--) { chain[(size_t)b * maxdepth + k] = c; c = parent[c]; }
+    for (int k = depth[b] - 1; k >= 0; k--) { h.chain[(size_t)b * maxdepth + k] = c; c = parent[c]; }
   }
   m.maxdepth = maxdepth;
-  std::vector<unsigned long long> submask(nb, 0ull), dofbody(std::max(m.nv, 1), 0ull);
+  h.submask.assign(nb, 0ull); h.dofbody.assign(std::max(m.nv, 1), 0ull);
   for (int d = 0; d < nb; d++)
     for (int a = 0; a < nb; a++)
-      if (ancmask[d] >> a & 1ull) submask[a] |= 1ull << d;
+      if (ancmask[d] >> a & 1ull) h.submask[a] |= 1ull << d;
   for (int b = 1; b < nb; b++)
     for (int i = 0; i < m.nv; i++)
-      if (dofmask[b] >> i & 1ull) dofbody[i] |= 1ull << b;
+      if (dofmask[b] >> i & 1ull) h.dofbody[i] |= 1ull << b;
   // compact kinematic records (fast path: every body has at most one joint)
-  std::vector<float> kinrec((size_t)nb * 16, 0.f);
-  int fastkin = 1;
+  h.kinrec.assign((size_t)nb * 16, 0.f);
+  m.fastkin = 1;
   {
-    const std::vector<int>& jn = s->mi["body_jntnum"]; const std::vector<int>& ja = s->mi["body_jntadr"];
-    const std::vector<double>& bp = s->mf["body_pos"]; const std::vector<double>& bq = s->mf["body_quat"];
-    const std::vector<double>& jp = s->mf["jnt_pos"]; const std::vector<double>& jax = s->mf["jnt_axis"];
-    const std::vector<double>& q0 = s->mf["qpos0"];
+    const std::vector<int>& jn = h.ints("body_jntnum"); const std::vector<int>& ja = h.ints("body_jntadr");
+    const std::vector<double>& bp = h.floats("body_pos"); const std::vector<double>& bq = h.floats("body_quat");
+    const std::vector<double>& jp = h.floats("jnt_pos"); const std::vector<double>& jax = h.floats("jnt_axis");
+    const std::vector<double>& q0 = h.floats("qpos0");
     for (int b = 0; b < nb; b++) {
-      if (jn[b] > 1) { fastkin = 0; break; }
-      float* r = kinrec.data() + 16 * b;
+      if (jn[b] > 1) { m.fastkin = 0; break; }
+      float* r = h.kinrec.data() + 16 * b;
       for (int k = 0; k < 3; k++) r[k] = (float)bp[3 * b + k];
       for (int k = 0; k < 4; k++) r[4 + k] = (float)bq[4 * b + k];
       int type = 0xff, j = 0, qa = 0;
       if (jn[b] == 1) {
-        j = ja[b]; type = s->mi["jnt_type"][j]; qa = s->mi["jnt_qposadr"][j];
+        j = ja[b]; type = h.ints("jnt_type")[j]; qa = h.ints("jnt_qposadr")[j];
         for (int k = 0; k < 3; k++) { r[8 + k] = (float)jp[3 * j + k]; r[12 + k] = (float)jax[3 * j + k]; }
         r[3] = (float)q0[qa];
       }
@@ -489,13 +488,12 @@ int b2_create(const B2ModelDesc* desc, int nworld, int ncon_per_world, int njmax
       memcpy(&r[15], &qa, 4);
     }
   }
-  m.fastkin = fastkin;
   // World pose (pos[3], mat[9], rbound) of a geom on a jointless child of the world body, in double from world 0's
   // model values: such geoms never move, so they are posed here once and shared by all worlds.
-  auto welded = [&](int g) { int b = s->mi["geom_bodyid"][g]; return b == 0 || (parent[b] == 0 && dofnum[b] == 0); };
+  auto welded = [&](int g) { int b = geom_bodyid[g]; return b == 0 || (parent[b] == 0 && dofnum[b] == 0); };
   auto world_pose = [&](int g, float* o) {
-    const std::vector<double>& bp = s->mf["body_pos"]; const std::vector<double>& bq = s->mf["body_quat"];
-    const std::vector<double>& gp = s->mf["geom_pos"]; const std::vector<double>& gq = s->mf["geom_quat"];
+    const std::vector<double>& bp = h.floats("body_pos"); const std::vector<double>& bq = h.floats("body_quat");
+    const std::vector<double>& gp = h.floats("geom_pos"); const std::vector<double>& gq = h.floats("geom_quat");
     auto qmul = [](const double* a, const double* b, double* r) {
       r[0] = a[0]*b[0] - a[1]*b[1] - a[2]*b[2] - a[3]*b[3];
       r[1] = a[0]*b[1] + a[1]*b[0] + a[2]*b[3] - a[3]*b[2];
@@ -507,7 +505,7 @@ int b2_create(const B2ModelDesc* desc, int nworld, int ncon_per_world, int njmax
       R[3] = 2*(q[1]*q[2] + q[0]*q[3]); R[4] = q[0]*q[0] - q[1]*q[1] + q[2]*q[2] - q[3]*q[3]; R[5] = 2*(q[2]*q[3] - q[0]*q[1]);
       R[6] = 2*(q[1]*q[3] - q[0]*q[2]); R[7] = 2*(q[2]*q[3] + q[0]*q[1]); R[8] = q[0]*q[0] - q[1]*q[1] - q[2]*q[2] + q[3]*q[3];
     };
-    const int b = s->mi["geom_bodyid"][g];
+    const int b = geom_bodyid[g];
     double Rb[9], q[4], R[9];
     q2m(&bq[4 * b], Rb);
     qmul(&bq[4 * b], &gq[4 * g], q);
@@ -517,282 +515,140 @@ int b2_create(const B2ModelDesc* desc, int nworld, int ncon_per_world, int njmax
     for (int i = 0; i < 3; i++)
       o[i] = (float)(bp[3 * b + i] + Rb[3 * i] * gp[3 * g] + Rb[3 * i + 1] * gp[3 * g + 1] + Rb[3 * i + 2] * gp[3 * g + 2]);
     for (int i = 0; i < 9; i++) o[3 + i] = (float)R[i];
-    o[12] = (float)s->mf["geom_rbound"][g];
+    o[12] = (float)h.floats("geom_rbound")[g];
   };
   // Pose slots of the collision geoms in shared memory.  Height fields welded to the world (a terrain has tens of
   // them) get no slot: their pose records live in global memory (fixed_pose, slot code -2 - index) - 56 bytes of
   // shared memory per field and per environment otherwise, and a pose computation per step.
-  std::vector<int> cslot(m.ngeom, -1), cgeom, fixed_geom;
+  std::vector<int> &cslot = h.cslot, &cgeom = h.cgeom, &fixed_geom = h.fixed_geom;
+  cslot.assign(m.ngeom, -1);
   {
     std::vector<char> second(m.ngeom, 0);
-    for (int p = 0; p < m.npair; p++) second[s->mi["pair_geom2"][p]] = 1;
+    for (int p = 0; p < m.npair; p++) second[pg2[p]] = 1;
     for (int p = 0; p < m.npair; p++) {
-      for (int g : {s->mi["pair_geom1"][p], s->mi["pair_geom2"][p]}) {
+      for (int g : {pg1[p], pg2[p]}) {
         if (cslot[g] != -1) continue;
-        if (s->mi["geom_type"][g] == G_HFIELD && !second[g] && welded(g)) { cslot[g] = -2 - (int)fixed_geom.size(); fixed_geom.push_back(g); }
+        if (gt[g] == G_HFIELD && !second[g] && welded(g)) { cslot[g] = -2 - (int)fixed_geom.size(); fixed_geom.push_back(g); }
         else { cslot[g] = (int)cgeom.size(); cgeom.push_back(g); }
       }
     }
   }
   m.nfixed = (int)fixed_geom.size();
-  std::vector<float> fixed_pose((size_t)std::max(m.nfixed, 1) * 16, 0.f);
-  for (int f = 0; f < m.nfixed; f++) world_pose(fixed_geom[f], fixed_pose.data() + 16 * (size_t)f);
+  h.fixed_pose.assign((size_t)std::max(m.nfixed, 1) * 16, 0.f);
+  for (int f = 0; f < m.nfixed; f++) world_pose(fixed_geom[f], h.fixed_pose.data() + 16 * (size_t)f);
   // grid-static collision set: static geoms never move, so their world poses are computed here once (in
   // double, from world 0's model values) and shared by all worlds; only the other geoms are posed per step
   m.nstatic = geti("nstatic");
-  m.ndyn = (int)s->mi["dyn_cgeom"].size();
-  std::vector<int> posegeom;
-  std::vector<float> static_pose((size_t)std::max(m.nstatic, 1) * 16, 0.f);
+  m.ndyn = (int)h.ints("dyn_cgeom").size();
+  h.static_pose.assign((size_t)std::max(m.nstatic, 1) * 16, 0.f);
   {
     std::vector<char> is_static(m.ngeom, 0);
-    const std::vector<int>& sg = s->mi["static_geom"];
-    if ((int)sg.size() != m.nstatic) { delete s; return fail("b2_create: static_geom / nstatic mismatch"); }
-    if (m.nstatic >= (1 << 20) || m.ndyn >= (1 << 11)) { delete s; return fail("b2_create: static grid too large"); }
+    const std::vector<int>& sg = h.ints("static_geom");
+    if ((int)sg.size() != m.nstatic) return fail("b2_create: static_geom / nstatic mismatch");
+    if (m.nstatic >= (1 << 20) || m.ndyn >= (1 << 11)) return fail("b2_create: static grid too large");
     for (int k = 0; k < m.nstatic; k++) {
-      int g = sg[k], b = s->mi["geom_bodyid"][g];
-      if (g < 0 || g >= m.ngeom || parent[b] != 0 || dofnum[b] != 0) {
-        delete s;
-        return fail("b2_create: grid-static geoms must sit on a jointless child of the world body");
-      }
+      int g = sg[k], b = geom_bodyid[g];
+      if (parent[b] != 0 || dofnum[b] != 0) return fail("b2_create: grid-static geoms must sit on a jointless child of the world body");
       is_static[g] = 1;
-      world_pose(g, static_pose.data() + 16 * (size_t)k);
+      world_pose(g, h.static_pose.data() + 16 * (size_t)k);
     }
     for (int g : fixed_geom) is_static[g] = 1;
-    for (int g = 0; g < m.ngeom; g++) if (!is_static[g]) posegeom.push_back(g);
-    m.nposegeom = (int)posegeom.size();
-    for (int g : s->mi["dyn_cgeom"]) {
-      if (g < 0 || g >= m.ngeom || is_static[g]) { delete s; return fail("b2_create: bad dyn_cgeom entry"); }
+    for (int g = 0; g < m.ngeom; g++) if (!is_static[g]) h.posegeom.push_back(g);
+    m.nposegeom = (int)h.posegeom.size();
+    for (int g : h.ints("dyn_cgeom")) {
+      if (is_static[g]) return fail("b2_create: bad dyn_cgeom entry");
       if (cslot[g] < 0) { cslot[g] = (int)cgeom.size(); cgeom.push_back(g); }
     }
     if (m.nstatic > 0) {
-      const std::vector<double>& gpar = s->mf["grid_params"];
-      if (gpar.size() != 5) { delete s; return fail("b2_create: grid_params must hold [x0, y0, cell, nx, ny]"); }
+      const std::vector<double>& gpar = h.floats("grid_params");
       m.grid_x0 = (float)gpar[0]; m.grid_y0 = (float)gpar[1]; m.grid_cell = (float)gpar[2];
       m.grid_nx = (int)gpar[3]; m.grid_ny = (int)gpar[4];
-      if ((int)s->mi["grid_start"].size() != m.grid_nx * m.grid_ny + 1 || (int)s->mi["static_cell0"].size() != 2 * m.nstatic) {
-        delete s;
+      if ((int)h.ints("grid_start").size() != m.grid_nx * m.grid_ny + 1)
         return fail("b2_create: static grid tables have inconsistent sizes");
-      }
     }
   }
   m.ncg = (int)cgeom.size();
   {  // every collision pair must have a narrowphase routine (primitives, or the convex routines of b2_convex.h)
-    const std::vector<int>& gt = s->mi["geom_type"];
     auto prim = [](int t) { return t == G_SPHERE || t == G_CAPSULE || t == G_BOX; };
     auto smooth = [](int t) { return t == G_ELLIPSOID || t == G_CYLINDER; };
     auto conv = [&](int t) { return prim(t) || t == G_MESH || smooth(t); };  // shapes the GJK/EPA routine takes (b2_convex.h)
-    const std::vector<int>& did = s->mi["geom_dataid"];
-    const int nmesh = (int)s->mi["mesh_vertnum"].size(), nhf = (int)s->mi["hfield_nrow"].size();
+    const std::vector<int>& did = h.ints("geom_dataid");
+    const std::vector<int> &mva = h.ints("mesh_vertadr"), &mvn = h.ints("mesh_vertnum");
+    const std::vector<int> &hadr = h.ints("hfield_adr"), &hnr = h.ints("hfield_nrow"), &hnc = h.ints("hfield_ncol");
+    const int nmesh = (int)mvn.size(), nhf = (int)hnr.size();
     for (int p = 0; p < m.npair; p++) {
-      int g1 = s->mi["pair_geom1"][p], g2 = s->mi["pair_geom2"][p];
+      int g1 = pg1[p], g2 = pg2[p];
       int t1 = gt[g1], t2 = gt[g2];
       bool ok = (t1 == G_PLANE && conv(t2)) || (t1 == G_HFIELD && conv(t2)) || (conv(t1) && conv(t2) && t1 <= t2);
-      if (t2 == G_MESH || t1 == G_HFIELD || smooth(t1) || smooth(t2)) s->has_convex = 1;
-      if (!ok) { delete s; return fail("b2_create: collision pair with an unsupported geom type combination"); }
+      if (t2 == G_MESH || t1 == G_HFIELD || smooth(t1) || smooth(t2)) h.has_convex = 1;
+      if (!ok) return fail("b2_create: collision pair with an unsupported geom type combination");
       for (int g : {g1, g2}) {
         int t = gt[g];
         if (t != G_MESH && t != G_HFIELD) continue;
         int id = g < (int)did.size() ? did[g] : -1;
-        if (id < 0 || id >= (t == G_MESH ? nmesh : nhf)) { delete s; return fail("b2_create: colliding mesh / hfield geom without asset data (geom_dataid)"); }
-        if (t == G_MESH && (s->mi["mesh_vertnum"][id] < 1 || (size_t)3 * (s->mi["mesh_vertadr"][id] + s->mi["mesh_vertnum"][id]) > s->mf["mesh_vert"].size())) {
-          delete s; return fail("b2_create: mesh vertex range outside mesh_vert");
-        }
-        if (t == G_HFIELD && (s->mi["hfield_nrow"][id] < 2 || s->mi["hfield_ncol"][id] < 2 || (size_t)4 * (id + 1) > s->mf["hfield_size"].size() ||
-                              (size_t)s->mi["hfield_adr"][id] + (size_t)s->mi["hfield_nrow"][id] * s->mi["hfield_ncol"][id] > s->mf["hfield_data"].size())) {
-          delete s; return fail("b2_create: hfield sample range outside hfield_data");
-        }
+        if (id < 0 || id >= (t == G_MESH ? nmesh : nhf)) return fail("b2_create: colliding mesh / hfield geom without asset data (geom_dataid)");
+        if (t == G_MESH && (mvn[id] < 1 || (size_t)3 * (mva[id] + mvn[id]) > h.floats("mesh_vert").size()))
+          return fail("b2_create: mesh vertex range outside mesh_vert");
+        if (t == G_HFIELD && (hnr[id] < 2 || hnc[id] < 2 || (size_t)4 * (id + 1) > h.floats("hfield_size").size() ||
+                              (size_t)hadr[id] + (size_t)hnr[id] * hnc[id] > h.floats("hfield_data").size()))
+          return fail("b2_create: hfield sample range outside hfield_data");
       }
     }
-    for (int g : s->mi["dyn_cgeom"]) {
-      if (!conv(gt[g])) { delete s; return fail("b2_create: unsupported dynamic geom type for the static grid"); }
-      if (gt[g] == G_MESH || smooth(gt[g])) s->has_convex = 1;
+    for (int g : h.ints("dyn_cgeom")) {
+      if (!conv(gt[g])) return fail("b2_create: unsupported dynamic geom type for the static grid");
+      if (gt[g] == G_MESH || smooth(gt[g])) h.has_convex = 1;
     }
-    for (int g : s->mi["static_geom"]) if (!prim(gt[g])) { delete s; return fail("b2_create: unsupported grid-static geom type"); }
+    for (int g : h.ints("static_geom")) if (!prim(gt[g])) return fail("b2_create: unsupported grid-static geom type");
   }
-  int rc = 0;
-#define UPI(field, key) rc |= dev_upload<int>(s, s->mi[key], &m.field)
-  UPI(body_parentid, "body_parentid"); UPI(body_rootid, "body_rootid"); UPI(body_jntadr, "body_jntadr");
-  UPI(body_jntnum, "body_jntnum"); UPI(body_dofadr, "body_dofadr"); UPI(body_dofnum, "body_dofnum");
-  UPI(jnt_type, "jnt_type"); UPI(jnt_qposadr, "jnt_qposadr"); UPI(jnt_dofadr, "jnt_dofadr");
-  UPI(jnt_bodyid, "jnt_bodyid"); UPI(jnt_limited, "jnt_limited"); UPI(dof_bodyid, "dof_bodyid");
-  UPI(dof_jntid, "dof_jntid"); UPI(dof_parentid, "dof_parentid"); UPI(geom_type, "geom_type");
-  UPI(geom_bodyid, "geom_bodyid"); UPI(geom_condim, "geom_condim"); UPI(geom_priority, "geom_priority");
-  UPI(site_bodyid, "site_bodyid"); UPI(actuator_trnid, "actuator_trnid");
-  UPI(actuator_ctrllimited, "actuator_ctrllimited"); UPI(actuator_forcelimited, "actuator_forcelimited");
-  UPI(pair_geom1, "pair_geom1"); UPI(pair_geom2, "pair_geom2"); UPI(sensor_objtype, "sensor_objtype");
-  UPI(geom_contype, "geom_contype"); UPI(geom_conaffinity, "geom_conaffinity"); UPI(dyn_cgeom, "dyn_cgeom");
-  UPI(static_geom, "static_geom"); UPI(static_cell0, "static_cell0"); UPI(grid_start, "grid_start");
-  UPI(grid_items, "grid_items");
-  UPI(geom_dataid, "geom_dataid"); UPI(mesh_vertadr, "mesh_vertadr"); UPI(mesh_vertnum, "mesh_vertnum");
-  UPI(hfield_adr, "hfield_adr"); UPI(hfield_nrow, "hfield_nrow"); UPI(hfield_ncol, "hfield_ncol");
-  UPI(sensor_objid, "sensor_objid"); UPI(sensor_reftype, "sensor_reftype");
-  UPI(sensor_refid, "sensor_refid"); UPI(sensor_intprm, "sensor_intprm"); UPI(sensor_adr, "sensor_adr");
-  UPI(sensor_dim, "sensor_dim");
-#undef UPI
-  rc |= dev_upload<int>(s, depth, &m.body_depth);
-  rc |= dev_upload<int>(s, chain, &m.body_chain);
-  rc |= dev_upload<unsigned long long>(s, dofmask, &m.body_dofmask);
-  rc |= dev_upload<unsigned long long>(s, ancmask, &m.body_ancmask);
-  rc |= dev_upload<unsigned long long>(s, submask, &m.body_submask);
-  rc |= dev_upload<unsigned long long>(s, dofbody, &m.dof_bodymask);
+  if (m.ncg >= 4096) return fail("b2_create: too many collision geoms");
+  h.pair_word.assign(std::max(m.npair, 1), 0u);
+  for (int p = 0; p < m.npair; p++)
+    h.pair_word[p] = (unsigned)std::max(cslot[pg1[p]], 0) | ((unsigned)std::max(cslot[pg2[p]], 0) << 12) |
+                     (gt[pg1[p]] == G_PLANE ? 0x80000000u : 0u) | (gt[pg1[p]] == G_HFIELD ? 0x40000000u : 0u);
   {
-    const float* kr = nullptr;
-    rc |= dev_upload<float>(s, kinrec, &kr);
-    m.kinrec = (const float4*)kr;
-  }
-  for (auto kv : {std::make_pair("mesh_vert", &m.mesh_vert), std::make_pair("hfield_size", &m.hfield_size),
-                  std::make_pair("hfield_data", &m.hfield_data)}) {
-    const std::vector<double>& h = s->mf[kv.first];
-    std::vector<float> hf(h.begin(), h.end());
-    rc |= dev_upload<float>(s, hf, kv.second);
-  }
-  rc |= dev_upload<int>(s, posegeom, &m.posegeom);
-  rc |= dev_upload<float>(s, static_pose, &m.static_pose);
-  {
-    if (m.ncg >= 4096) { b2_destroy(s); return fail("b2_create: too many collision geoms"); }
-    std::vector<unsigned> pw(std::max(m.npair, 1), 0u);
-    for (int p = 0; p < m.npair; p++) {
-      int g1 = s->mi["pair_geom1"][p], g2 = s->mi["pair_geom2"][p];
-      pw[p] = (unsigned)std::max(cslot[g1], 0) | ((unsigned)std::max(cslot[g2], 0) << 12) | (s->mi["geom_type"][g1] == G_PLANE ? 0x80000000u : 0u) |
-              (s->mi["geom_type"][g1] == G_HFIELD ? 0x40000000u : 0u);
-    }
-    rc |= dev_upload<unsigned>(s, pw, &m.pair_word);
     // height-field pairs grouped by field: the kernel first finds the fields under the robot, then tests only
     // their pairs (a terrain is a grid of fields; the flat pair table would test every one of them)
-    std::vector<int> hf_geom, hf_slot, hf_start, hf_pairs, hfd, nh;  // (hf_slot: pose slot, or -2 - index into fixed_pose)
     std::vector<std::vector<int>> per;
-    std::vector<float> box;
     for (int p = 0; p < m.npair; p++) {
-      int g1 = s->mi["pair_geom1"][p], g2 = s->mi["pair_geom2"][p];
-      if (s->mi["geom_type"][g1] != G_HFIELD) { nh.push_back(p); continue; }
-      size_t h = std::find(hf_geom.begin(), hf_geom.end(), g1) - hf_geom.begin();
-      if (h == hf_geom.size()) {
-        hf_geom.push_back(g1); hf_slot.push_back(cslot[g1]); per.emplace_back();
-        const int id = s->mi["geom_dataid"][g1];
-        for (int k = 0; k < 4; k++) box.push_back((float)s->mf["hfield_size"][4 * (size_t)id + k]);
+      int g1 = pg1[p], g2 = pg2[p];
+      if (gt[g1] != G_HFIELD) { h.nh.push_back(p); continue; }
+      size_t f = std::find(h.hf_geom.begin(), h.hf_geom.end(), g1) - h.hf_geom.begin();
+      if (f == h.hf_geom.size()) {
+        h.hf_geom.push_back(g1); h.hf_slot.push_back(cslot[g1]); per.emplace_back();
+        const int id = h.ints("geom_dataid")[g1];
+        for (int k = 0; k < 4; k++) h.hf_box.push_back((float)h.floats("hfield_size")[4 * (size_t)id + k]);
       }
-      per[h].push_back(p);
-      if (std::find(hfd.begin(), hfd.end(), cslot[g2]) == hfd.end()) hfd.push_back(cslot[g2]);
+      per[f].push_back(p);
+      if (std::find(h.hfd.begin(), h.hfd.end(), cslot[g2]) == h.hfd.end()) h.hfd.push_back(cslot[g2]);
     }
-    m.nhf = (int)hf_geom.size(); m.nhfd = (int)hfd.size(); m.n_nhpair = m.npair;
-    m.hfl_slot = m.hfl_geom = m.hfl_start = m.hfl_pairs = m.hfd_slot = m.nh_pairs = nullptr; m.hfl_box = nullptr;
+    m.nhf = (int)h.hf_geom.size(); m.nhfd = (int)h.hfd.size(); m.n_nhpair = m.npair;
     if (m.nhf > 0) {
-      for (auto& v : per) { hf_start.push_back((int)hf_pairs.size()); hf_pairs.insert(hf_pairs.end(), v.begin(), v.end()); }
-      hf_start.push_back((int)hf_pairs.size());
-      m.n_nhpair = (int)nh.size();
-      if (nh.empty()) nh.push_back(0);
-      const float* bp = nullptr;
-      rc |= dev_upload<int>(s, hf_slot, &m.hfl_slot); rc |= dev_upload<int>(s, hf_start, &m.hfl_start);
-      rc |= dev_upload<int>(s, hf_geom, &m.hfl_geom);
-      rc |= dev_upload<int>(s, hf_pairs, &m.hfl_pairs); rc |= dev_upload<int>(s, hfd, &m.hfd_slot);
-      rc |= dev_upload<int>(s, nh, &m.nh_pairs); rc |= dev_upload<float>(s, box, &bp);
-      m.hfl_box = (const float4*)bp;
+      for (auto& v : per) { h.hf_start.push_back((int)h.hf_pairs.size()); h.hf_pairs.insert(h.hf_pairs.end(), v.begin(), v.end()); }
+      h.hf_start.push_back((int)h.hf_pairs.size());
+      m.n_nhpair = (int)h.nh.size();
+      if (h.nh.empty()) h.nh.push_back(0);
     }
   }
-  rc |= dev_upload<int>(s, cslot, &m.geom_cslot);
-  rc |= dev_upload<float>(s, fixed_pose, &m.fixed_pose);
   if (fixed_geom.empty()) fixed_geom.push_back(0);
-  rc |= dev_upload<int>(s, fixed_geom, &m.fixed_geom);
-  rc |= dev_upload<int>(s, cgeom, &m.cgeom);
-  {
-    // schedules of the bottom-up blocked factorisation (b2_kernel.cuh: ldl_factor)
-    std::vector<unsigned> dense, sparse;
-    b2_build_ldl_schedules(m.nv, s->mi["dof_parentid"].data(), dense, sparse, m.ldl_start);
-    m.ldl_nsparse = (int)sparse.size();
-    rc |= dev_upload<unsigned>(s, dense, &m.ldl_dense);
-    rc |= dev_upload<unsigned>(s, sparse, &m.ldl_sparse);
-  }
-  if (rc) { b2_destroy(s); return 1; }
+  // schedules of the bottom-up blocked factorisation (b2_kernel.cuh: ldl_factor)
+  b2_build_ldl_schedules(m.nv, h.ints("dof_parentid").data(), h.ldl_dense, h.ldl_sparse, m.ldl_start);
+  m.ldl_nsparse = (int)h.ldl_sparse.size();
   // supported sensor set: contact sensors with data in {found,force,dist,pos,normal}, reduce none/netforce
   for (int i = 0; i < m.nsensor; i++) {
-    int ds = s->mi["sensor_intprm"][3 * i], rd = s->mi["sensor_intprm"][3 * i + 1];
-    if ((ds & ~(1 | 2 | 8 | 16 | 32)) || (rd != 0 && rd != 3)) {
-      b2_destroy(s);
+    int ds = h.ints("sensor_intprm")[3 * i], rd = h.ints("sensor_intprm")[3 * i + 1];
+    if ((ds & ~(1 | 2 | 8 | 16 | 32)) || (rd != 0 && rd != 3))
       return fail("b2_create: contact sensor data/reduce combination not implemented");
-    }
   }
-  // int model fields visible to callers
-  auto add_imodel = [&](const char* name, const int* p, int n) {
-    Field f; f.name = name; f.ptr = (void*)p; f.dtype = B2_I32; f.ndim = 1; f.shape[0] = n; f.stride[0] = 1; f.n = n;
-    s->model_fields.push_back(f);
-  };
-  add_imodel("geom_bodyid", m.geom_bodyid, m.ngeom); add_imodel("site_bodyid", m.site_bodyid, m.nsite);
-  add_imodel("body_parentid", m.body_parentid, nb); add_imodel("body_rootid", m.body_rootid, nb);
-  add_imodel("jnt_type", m.jnt_type, m.njnt); add_imodel("jnt_qposadr", m.jnt_qposadr, m.njnt);
-  add_imodel("jnt_dofadr", m.jnt_dofadr, m.njnt); add_imodel("dof_bodyid", m.dof_bodyid, m.nv);
-  add_imodel("geom_type", m.geom_type, m.ngeom); add_imodel("geom_condim", m.geom_condim, m.ngeom);
-  add_imodel("geom_priority", m.geom_priority, m.ngeom);
-  add_imodel("actuator_trnid", m.actuator_trnid, m.nu);
-
-  // ---- float model arrays (fp32 on device; shared by all worlds until expanded) -----------------
-  for (const ShapeSpec& sp : kModelShapes) {
-    const std::vector<double>& h = s->mf[sp.name];
-    std::vector<float> hf(h.begin(), h.end());
-    const float* p = nullptr;
-    if (dev_upload<float>(s, hf, &p)) { b2_destroy(s); return 1; }
-    FArr* fa = model_farr(m, sp.name);
-    fa->p = p; fa->stride = 0; fa->n = (int)hf.size();
-    Field f; f.name = sp.name; f.ptr = (void*)p; f.dtype = B2_F32; f.farr = fa; f.n = (int64_t)hf.size();
-    if (sp.second > 0) {
-      f.ndim = 3; f.shape[0] = nworld; f.shape[1] = (int64_t)hf.size() / sp.second; f.shape[2] = sp.second;
-      f.stride[0] = 0; f.stride[1] = sp.second; f.stride[2] = 1;
-    } else {
-      f.ndim = 2; f.shape[0] = nworld; f.shape[1] = (int64_t)hf.size(); f.stride[0] = 0; f.stride[1] = 1;
-    }
-    s->model_fields.push_back(f);
-  }
-
-  // ---- data -------------------------------------------------------------------------------------
-  DevData& d = s->hd;
-  memset(&d, 0, sizeof(d));
-  d.nworld = nworld;
-  int nq = m.nq, nv = m.nv, nu = m.nu, ng = m.ngeom, ns = m.nsite, mc = m.maxcon;
-  rc = 0;
-  rc |= add_data(s, "qpos", &d.qpos, nq); rc |= add_data(s, "qvel", &d.qvel, nv);
-  rc |= add_data(s, "ctrl", &d.ctrl, nu); rc |= add_data(s, "qacc_warmstart", &d.qacc_warmstart, nv);
-  rc |= add_data(s, "qfrc_applied", &d.qfrc_applied, nv);
-  rc |= add_data(s, "xfrc_applied", &d.xfrc_applied, 6 * nb, 6);
-  rc |= add_data(s, "act", &d.act, 0);
-  rc |= add_data(s, "qacc", &d.qacc, nv); rc |= add_data(s, "xpos", &d.xpos, 3 * nb, 3);
-  rc |= add_data(s, "xquat", &d.xquat, 4 * nb, 4); rc |= add_data(s, "xmat", &d.xmat, 9 * nb, 9);
-  rc |= add_data(s, "xipos", &d.xipos, 3 * nb, 3); rc |= add_data(s, "subtree_com", &d.subtree_com, 3 * nb, 3);
-  rc |= add_data(s, "cvel", &d.cvel, 6 * nb, 6); rc |= add_data(s, "geom_xpos", &d.geom_xpos, 3 * ng, 3);
-  rc |= add_data(s, "geom_xmat", &d.geom_xmat, 9 * ng, 9); rc |= add_data(s, "site_xpos", &d.site_xpos, 3 * ns, 3);
-  rc |= add_data(s, "site_xmat", &d.site_xmat, 9 * ns, 9);
-  rc |= add_data(s, "link_vel_w", &d.link_vel_w, 6 * nb, 6); rc |= add_data(s, "com_vel_w", &d.com_vel_w, 6 * nb, 6);
-  rc |= add_data(s, "link_state_b", &d.link_state_b, 10 * nb, 10);
-  rc |= add_data(s, "sensordata", &d.sensordata, m.nsensordata);
-  rc |= add_data(s, "actuator_force", &d.actuator_force, nu); rc |= add_data(s, "time", &d.time, 1);
-  rc |= add_data(s, "qfrc_bias", &d.qfrc_bias, nv); rc |= add_data(s, "qfrc_smooth", &d.qfrc_smooth, nv);
-  rc |= add_data(s, "qacc_smooth", &d.qacc_smooth, nv);
-  rc |= add_data(s, "qfrc_constraint", &d.qfrc_constraint, nv);
-  rc |= add_data(s, "qM", &d.qM, nv * nv, nv);
-  rc |= add_data(s, "qM_packed", &d.qM_packed, m.ntri);
-  rc |= add_data(s, "qacc_smooth_prev", &d.qacc_smooth_prev, nv);
-  rc |= add_data(s, "ctrl_prev", &d.ctrl_prev, nu);
-  rc |= add_data(s, "contact_dist", &d.contact_dist, mc); rc |= add_data(s, "contact_pos", &d.contact_pos, 3 * mc, 3);
-  rc |= add_data(s, "contact_frame", &d.contact_frame, 9 * mc, 9);
-  rc |= add_data(s, "contact_force", &d.contact_force, 3 * mc, 3);
-  rc |= add_data(s, "solver_cost", &d.solver_cost, 1);
-  rc |= add_idata(s, "ncon", &d.ncon, 1); rc |= add_idata(s, "nefc", &d.nefc, 1);
-  rc |= add_idata(s, "solver_niter", &d.solver_niter, 1);
-  rc |= add_idata(s, "contact_geom", &d.contact_geom, 2 * mc, 2);
-  rc |= add_idata(s, "overflow", &d.overflow, 1);
-  rc |= add_idata(s, "solver_nd", &d.solver_nd, 1);
-  rc |= add_idata(s, "solver_nls", &d.solver_nls, 1);  // line-search derivative evaluations of the last step (diagnostic)
-  if (rc) { b2_destroy(s); return 1; }
-  // time is exposed as a 1-D (nworld,) tensor
-  for (Field& f : s->data_fields)
-    if (f.name == "time" || f.name == "solver_cost") { f.ndim = 1; }
 
   // ---- shared-memory layout (floats per environment) -------------------------------------------
+  int nq = m.nq, nv = m.nv, nu = m.nu, mc = m.maxcon;
   Layout& L = m.lay;
   int off = 0;
   auto alloc = [&](int n) { int o = off; off += pad4(std::max(n, 1)); return o; };
   L.maxcon = mc;
   L.nlimcap = pad4(std::max(m.njnt, 1));
   L.maxpair = m.nstatic > 0 ? 256 : 128;
-  L.qpos = alloc(d.qpos.stride); L.qvel = alloc(d.qvel.stride); L.qacc_ws = alloc(d.qacc_warmstart.stride);
+  L.qpos = alloc(nq); L.qvel = alloc(nv); L.qacc_ws = alloc(nv);  // (one Data row each: add_data pads rows alike)
   L.cdof = alloc(7 * nv);
   int hsize = std::max(m.ntri, pad4(GP * m.ncg) + L.maxpair);
   L.H = alloc(hsize); L.gpose = L.H; L.pairlist = L.H + pad4(GP * m.ncg);
@@ -828,72 +684,177 @@ int b2_create(const B2ModelDesc* desc, int nworld, int ncon_per_world, int njmax
   int endB = off;
   // the lane-distributed height-field narrowphase keeps its owner records and its queue in the (then unused)
   // solver regions from gV on
-  if (!s->mf["hfield_data"].empty()) endB = std::max(endB, L.gV + HF_SCRATCH);
+  if (!h.floats("hfield_data").empty()) endB = std::max(endB, L.gV + HF_SCRATCH);
   L.total = pad4(std::max(endA, endB));
   if (L.ndcap == 0) L.Mred = L.H;  // never used
-  s->smem_bytes = sizeof(float) * ((size_t)L.total * B2_WARPS_PER_CTA + pad4(m.ldl_nsparse + 18));
-  if (s->smem_bytes > 227 * 1024) {
-    b2_destroy(s);
-    return fail("b2_create: model too large for the per-environment shared-memory block");
+  h.smem_bytes = sizeof(float) * ((size_t)L.total * B2_WARPS_PER_CTA + pad4(m.ldl_nsparse + 18));
+  if (h.smem_bytes > 227 * 1024) return fail("b2_create: model too large for the per-environment shared-memory block");
+  return 0;
+}
+
+// The device stage of b2_create: uploads the model, allocates the Data arrays and runs the initial forward pass.
+static int setup_device(b2_sim* s, const HostModel& h) {
+  DevModel& m = s->hm;
+  m = h.m;
+  s->has_convex = h.has_convex;
+  s->smem_bytes = h.smem_bytes;
+  int rc = 0;
+  for (const IntArray& a : int_arrays(h.z)) {
+    rc |= dev_upload(s, h.ints(a.name), &(m.*a.member));
+    if (!a.visible) continue;
+    Field f; f.name = a.name; f.ptr = (void*)(m.*a.member); f.dtype = B2_I32; f.shape[0] = f.n = a.n; f.stride[0] = 1;
+    s->model_fields.push_back(f);
   }
+  const float *kinrec = nullptr, *hf_box = nullptr;
+  rc |= dev_upload(s, h.depth, &m.body_depth);
+  rc |= dev_upload(s, h.chain, &m.body_chain);
+  rc |= dev_upload(s, h.dofmask, &m.body_dofmask);
+  rc |= dev_upload(s, h.ancmask, &m.body_ancmask);
+  rc |= dev_upload(s, h.submask, &m.body_submask);
+  rc |= dev_upload(s, h.dofbody, &m.dof_bodymask);
+  rc |= dev_upload(s, h.kinrec, &kinrec);
+  rc |= dev_upload(s, to_float(h.floats("mesh_vert")), &m.mesh_vert);
+  rc |= dev_upload(s, to_float(h.floats("hfield_size")), &m.hfield_size);
+  rc |= dev_upload(s, to_float(h.floats("hfield_data")), &m.hfield_data);
+  rc |= dev_upload(s, h.posegeom, &m.posegeom);
+  rc |= dev_upload(s, h.static_pose, &m.static_pose);
+  rc |= dev_upload(s, h.pair_word, &m.pair_word);
+  if (m.nhf > 0) {
+    rc |= dev_upload(s, h.hf_slot, &m.hfl_slot); rc |= dev_upload(s, h.hf_start, &m.hfl_start);
+    rc |= dev_upload(s, h.hf_geom, &m.hfl_geom);
+    rc |= dev_upload(s, h.hf_pairs, &m.hfl_pairs); rc |= dev_upload(s, h.hfd, &m.hfd_slot);
+    rc |= dev_upload(s, h.nh, &m.nh_pairs); rc |= dev_upload(s, h.hf_box, &hf_box);
+  }
+  rc |= dev_upload(s, h.cslot, &m.geom_cslot);
+  rc |= dev_upload(s, h.fixed_pose, &m.fixed_pose);
+  rc |= dev_upload(s, h.fixed_geom, &m.fixed_geom);
+  rc |= dev_upload(s, h.cgeom, &m.cgeom);
+  rc |= dev_upload(s, h.ldl_dense, &m.ldl_dense);
+  rc |= dev_upload(s, h.ldl_sparse, &m.ldl_sparse);
+  if (rc) return 1;
+  m.kinrec = (const float4*)kinrec;
+  m.hfl_box = (const float4*)hf_box;
+
+  // ---- float model arrays (fp32 on device; shared by all worlds until expanded) -----------------
+  for (const FloatArray& a : float_arrays(h.z)) {
+    FArr& fa = m.*a.member;
+    if (dev_upload(s, to_float(h.floats(a.name)), &fa.p)) return 1;
+    fa.stride = 0; fa.n = (int)a.n;
+    Field f; f.name = a.name; f.ptr = (void*)fa.p; f.dtype = B2_F32; f.farr = &fa; f.n = a.n;
+    f.shape[0] = s->nworld; f.stride[0] = 0;
+    if (a.width > 1) {
+      f.ndim = 3; f.shape[1] = a.n / a.width; f.shape[2] = a.width; f.stride[1] = a.width; f.stride[2] = 1;
+    } else {
+      f.ndim = 2; f.shape[1] = a.n; f.stride[1] = 1;
+    }
+    s->model_fields.push_back(f);
+  }
+
+  // ---- data -------------------------------------------------------------------------------------
+  DevData& d = s->hd;
+  memset(&d, 0, sizeof(d));
+  d.nworld = s->nworld;
+  const int nq = m.nq, nv = m.nv, nu = m.nu, nb = m.nbody, ng = m.ngeom, ns = m.nsite, mc = m.maxcon;
+  rc |= add_data(s, "qpos", &d.qpos, {nq}); rc |= add_data(s, "qvel", &d.qvel, {nv});
+  rc |= add_data(s, "ctrl", &d.ctrl, {nu}); rc |= add_data(s, "qacc_warmstart", &d.qacc_warmstart, {nv});
+  rc |= add_data(s, "qfrc_applied", &d.qfrc_applied, {nv});
+  rc |= add_data(s, "xfrc_applied", &d.xfrc_applied, {nb, 6});
+  rc |= add_data(s, "act", &d.act, {0});
+  rc |= add_data(s, "qacc", &d.qacc, {nv}); rc |= add_data(s, "xpos", &d.xpos, {nb, 3});
+  rc |= add_data(s, "xquat", &d.xquat, {nb, 4}); rc |= add_data(s, "xmat", &d.xmat, {nb, 3, 3});
+  rc |= add_data(s, "xipos", &d.xipos, {nb, 3}); rc |= add_data(s, "subtree_com", &d.subtree_com, {nb, 3});
+  rc |= add_data(s, "cvel", &d.cvel, {nb, 6}); rc |= add_data(s, "geom_xpos", &d.geom_xpos, {ng, 3});
+  rc |= add_data(s, "geom_xmat", &d.geom_xmat, {ng, 3, 3}); rc |= add_data(s, "site_xpos", &d.site_xpos, {ns, 3});
+  rc |= add_data(s, "site_xmat", &d.site_xmat, {ns, 3, 3});
+  rc |= add_data(s, "link_vel_w", &d.link_vel_w, {nb, 6}); rc |= add_data(s, "com_vel_w", &d.com_vel_w, {nb, 6});
+  rc |= add_data(s, "link_state_b", &d.link_state_b, {nb, 10});
+  rc |= add_data(s, "sensordata", &d.sensordata, {m.nsensordata});
+  rc |= add_data(s, "actuator_force", &d.actuator_force, {nu}); rc |= add_data(s, "time", &d.time, {});
+  rc |= add_data(s, "qfrc_bias", &d.qfrc_bias, {nv}); rc |= add_data(s, "qfrc_smooth", &d.qfrc_smooth, {nv});
+  rc |= add_data(s, "qacc_smooth", &d.qacc_smooth, {nv});
+  rc |= add_data(s, "qfrc_constraint", &d.qfrc_constraint, {nv});
+  rc |= add_data(s, "qM", &d.qM, {nv, nv});
+  rc |= add_data(s, "qM_packed", &d.qM_packed, {m.ntri});
+  rc |= add_data(s, "qacc_smooth_prev", &d.qacc_smooth_prev, {nv});
+  rc |= add_data(s, "ctrl_prev", &d.ctrl_prev, {nu});
+  rc |= add_data(s, "contact_dist", &d.contact_dist, {mc}); rc |= add_data(s, "contact_pos", &d.contact_pos, {mc, 3});
+  rc |= add_data(s, "contact_frame", &d.contact_frame, {mc, 3, 3});
+  rc |= add_data(s, "contact_force", &d.contact_force, {mc, 3});
+  rc |= add_data(s, "solver_cost", &d.solver_cost, {});
+  rc |= add_data(s, "ncon", &d.ncon, {}); rc |= add_data(s, "nefc", &d.nefc, {});
+  rc |= add_data(s, "solver_niter", &d.solver_niter, {});
+  rc |= add_data(s, "contact_geom", &d.contact_geom, {mc, 2});
+  rc |= add_data(s, "overflow", &d.overflow, {});
+  rc |= add_data(s, "solver_nd", &d.solver_nd, {});
+  rc |= add_data(s, "solver_nls", &d.solver_nls, {});  // line-search derivative evaluations of the last step (diagnostic)
+  if (rc) return 1;
+
   {
     // The attribute is per function and per device, not per sim: only ever raise it, so that an earlier,
     // larger sim in the same process keeps launching after a smaller one is created.
     static size_t dev_max[64] = {0};
-    if (s->smem_bytes > dev_max[cuda_device & 63]) {
+    if (s->smem_bytes > dev_max[s->device & 63]) {
       cudaError_t e1 = cudaFuncSetAttribute(b2_step_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->smem_bytes);
       cudaError_t e2 = cudaFuncSetAttribute(b2_step_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->smem_bytes);
       if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(b2_step_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->smem_bytes);
       if (e2 == cudaSuccess) e2 = cudaFuncSetAttribute(b2_step_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->smem_bytes);
-      if (e1 != cudaSuccess || e2 != cudaSuccess) {
-        b2_destroy(s);
+      if (e1 != cudaSuccess || e2 != cudaSuccess)
         return fail(std::string("cudaFuncSetAttribute(max dynamic smem): ") + cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
-      }
-      dev_max[cuda_device & 63] = s->smem_bytes;
+      dev_max[s->device & 63] = s->smem_bytes;
     }
   }
   {
     void* p = nullptr;
-    if (cudaMalloc(&p, sizeof(int) * (size_t)nworld) != cudaSuccess) { b2_destroy(s); return fail("cudaMalloc(order)"); }
+    if (cudaMalloc(&p, sizeof(int) * (size_t)s->nworld) != cudaSuccess) return fail("cudaMalloc(order)");
     s->allocs.push_back(p);
     s->order = (int*)p;
-    for (int h = 0; h < B2_PARTITIONS; h++) {
-      if (cudaStreamCreateWithFlags(&s->side[h], cudaStreamNonBlocking) != cudaSuccess ||
-          cudaEventCreateWithFlags(&s->ev_join[h], cudaEventDisableTiming) != cudaSuccess) {
-        b2_destroy(s);
+    for (int k = 0; k < B2_PARTITIONS; k++)
+      if (cudaStreamCreateWithFlags(&s->side[k], cudaStreamNonBlocking) != cudaSuccess ||
+          cudaEventCreateWithFlags(&s->ev_join[k], cudaEventDisableTiming) != cudaSuccess)
         return fail("b2_create: stream/event creation failed");
-      }
-    }
-    if (cudaEventCreateWithFlags(&s->ev_fork, cudaEventDisableTiming) != cudaSuccess) { b2_destroy(s); return fail("event"); }
+    if (cudaEventCreateWithFlags(&s->ev_fork, cudaEventDisableTiming) != cudaSuccess) return fail("event");
   }
   // qpos <- qpos0 in every world, then one forward pass so all derived fields are valid
-  {
-    long long total = (long long)nworld * nq;
-    b2_init_rows_kernel<<<(unsigned)((total + 255) / 256), 256>>>(d.qpos.p, d.qpos.stride, m.qpos0.p, nq, nworld);
+  const int nworld = s->nworld;
+  long long total = (long long)nworld * nq;
+  b2_init_rows_kernel<<<(unsigned)((total + 255) / 256), 256>>>(d.qpos.p, d.qpos.stride, m.qpos0.p, nq, nworld);
+  s->launches++;
+  if (m.nstatic > 0) {
+    long long tot = (long long)nworld * m.nstatic;
+    b2_static_rows_kernel<<<(unsigned)((tot + 255) / 256), 256>>>(d.geom_xpos.p, d.geom_xpos.stride, d.geom_xmat.p,
+                                                                   d.geom_xmat.stride, m.static_pose, m.static_geom,
+                                                                   m.nstatic, nworld);
     s->launches++;
-    if (m.nstatic > 0) {
-      long long tot = (long long)nworld * m.nstatic;
-      b2_static_rows_kernel<<<(unsigned)((tot + 255) / 256), 256>>>(d.geom_xpos.p, d.geom_xpos.stride, d.geom_xmat.p,
-                                                                     d.geom_xmat.stride, m.static_pose, m.static_geom,
-                                                                     m.nstatic, nworld);
-      s->launches++;
-    }
-    if (m.nfixed > 0) {
-      long long tot = (long long)nworld * m.nfixed;
-      b2_static_rows_kernel<<<(unsigned)((tot + 255) / 256), 256>>>(d.geom_xpos.p, d.geom_xpos.stride, d.geom_xmat.p,
-                                                                     d.geom_xmat.stride, m.fixed_pose, m.fixed_geom,
-                                                                     m.nfixed, nworld);
-      s->launches++;
-    }
-    if (launch(s, false, 0)) { b2_destroy(s); return 1; }
-    cudaError_t e = cudaDeviceSynchronize();
-    if (e != cudaSuccess) {
-      std::string msg = std::string("b2_create: initial forward failed: ") + cudaGetErrorString(e);
-      b2_destroy(s);
-      return fail(msg);
-    }
   }
-  *out = s;
+  if (m.nfixed > 0) {
+    long long tot = (long long)nworld * m.nfixed;
+    b2_static_rows_kernel<<<(unsigned)((tot + 255) / 256), 256>>>(d.geom_xpos.p, d.geom_xpos.stride, d.geom_xmat.p,
+                                                                   d.geom_xmat.stride, m.fixed_pose, m.fixed_geom,
+                                                                   m.nfixed, nworld);
+    s->launches++;
+  }
+  if (launch(s, false, 0)) return 1;
+  cudaError_t e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) return fail(std::string("b2_create: initial forward failed: ") + cudaGetErrorString(e));
+  return 0;
+}
+
+int b2_create(const B2ModelDesc* desc, int nworld, int ncon_per_world, int njmax, int cuda_device,
+              b2_sim** out) {
+  if (!desc || !out || nworld <= 0) return fail("b2_create: bad arguments");
+  HostModel h;
+  if (plan_model(desc, ncon_per_world, njmax, h)) return 1;
+  // (every check that can reject the descriptor has run: without a GPU, a malformed model reports what is wrong)
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+    return fail("b2_create: no CUDA device available (this library has no CPU path)");
+  if (cuda_device < 0 || cuda_device >= ndev) return fail("b2_create: bad cuda_device");
+  DeviceGuard guard(cuda_device);
+  std::unique_ptr<b2_sim, decltype(&b2_destroy)> s(new b2_sim(), b2_destroy);
+  s->device = cuda_device;
+  s->nworld = nworld;
+  if (setup_device(s.get(), h)) return 1;
+  *out = s.release();
   return 0;
 }
 

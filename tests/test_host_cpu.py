@@ -152,13 +152,15 @@ def test_shard_range():
 
 
 def test_b2_create_rejects_malformed_model_tables(g1_model):
-  """The descriptor is validated on the host before any device work: wrong sizes and out-of-range indices are
-  refused with a message (no compute happens here; on a CPU box a valid table ends at 'no CUDA device')."""
+  """The descriptor is checked on the host before any device work: wrong sizes, out-of-range indices and models the
+  engine does not support are refused with a message (no compute happens here; on a CPU box a valid table ends at
+  'no CUDA device')."""
   import copy
   import ctypes
 
   import numpy as np
 
+  from mjlab_b200.asset_zoo import load_compiled
   from mjlab_b200.sim import native
 
   lib = native.load_library()
@@ -173,17 +175,35 @@ def test_b2_create_rejects_malformed_model_tables(g1_model):
       lib.b2_destroy(h)
     return rc, msg
 
-  rc, msg = create(g1_model)
-  assert rc == 0 or "no CUDA device" in msg  # the unmodified table passes validation
+  def set_at(index, value):
+    def mod(a):
+      a = a.copy()
+      a[index] = value
+      return a
+    return mod
+
+  terrain = load_compiled("go1_rough")
+  for model in (g1_model, terrain):
+    rc, msg = create(model)
+    assert rc == 0 or "no CUDA device" in msg  # the unmodified table passes validation
+  # a terrain geom moved onto the first body with a joint (the trunk)
+  trunk = int(np.flatnonzero(np.asarray(terrain.arrays["body_jntnum"]))[0])
+  static_on_trunk = set_at(int(np.asarray(terrain.arrays["static_geom"])[0]), trunk)
   cases = [
-    ("dof_parentid", lambda a: a[:-1], "has 34 elements, expected 35"),
-    ("pair_geom1", lambda a: np.where(np.arange(len(a)) == 3, 999, a).astype(np.int32), "index out of range"),
-    ("geom_size", lambda a: a[:-1], "'geom_size' has"),
-    ("body_parentid", lambda a: np.where(np.arange(len(a)) == 2, 5, a).astype(np.int32), "parents must precede children"),
+    (g1_model, "dof_parentid", lambda a: a[:-1], "has 34 elements, expected 35"),
+    (g1_model, "pair_geom1", lambda a: np.where(np.arange(len(a)) == 3, 999, a).astype(np.int32), "index out of range"),
+    (g1_model, "geom_size", lambda a: a[:-1], "'geom_size' has"),
+    (g1_model, "body_parentid", lambda a: np.where(np.arange(len(a)) == 2, 5, a).astype(np.int32), "parents must precede children"),
+    # the checks below follow the table checks; none of them needs a device
+    (g1_model, "pair_geom2", set_at(0, 0), "unsupported geom type combination"),  # the floor (geom 0) against itself
+    (g1_model, "opt_solver", lambda a: np.zeros_like(a), "solver must be Newton or CG"),
+    (g1_model, "opt_cone", lambda a: np.ones_like(a), "only pyramidal cones are supported"),
+    (g1_model, "sensor_intprm", set_at((0, 0), 1 | 4), "contact sensor data/reduce combination not implemented"),
+    (terrain, "geom_bodyid", static_on_trunk, "grid-static geoms must sit on a jointless child of the world body"),
   ]
-  for field, mod, expect in cases:
-    m2 = copy.deepcopy(g1_model)
-    m2.arrays[field] = np.ascontiguousarray(mod(np.asarray(g1_model.arrays[field])))
+  for model, field, mod, expect in cases:
+    m2 = copy.deepcopy(model)
+    m2.arrays[field] = np.ascontiguousarray(mod(np.asarray(model.arrays[field])))
     rc, msg = create(m2)
     assert rc != 0 and expect in msg, (field, msg)
 

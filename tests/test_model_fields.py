@@ -15,8 +15,9 @@ from oracle.oracle import Oracle
 from test_kernel_emul import EmulSim, _load
 from util import _quat_mul, load_oracle, make_states, relerr
 
-# kModelShapes (b2sim.cu) minus geom_rgba (never read) and dof_frictionloss (the compiler refuses friction loss and
-# the kernel has no friction-loss rows)
+# The library's float model fields (B2_MODEL_FARRAYS in b2_types.h) minus geom_rgba (never read) and dof_frictionloss
+# (the compiler refuses friction loss and the kernel has no friction-loss rows); test_fields_are_the_float_model_fields
+# holds the two lists together.
 FIELDS = [
   "body_pos", "body_quat", "body_ipos", "body_iquat", "body_mass", "body_subtreemass", "body_inertia",
   "body_invweight0", "jnt_pos", "jnt_axis", "jnt_range", "jnt_solref", "jnt_solimp", "jnt_margin", "jnt_stiffness",
@@ -275,6 +276,24 @@ def _baseline(lib, m, n, seed, kind, name):
     _baselines[key] = _emul_run(sim, states(m, n, seed, kind))
     sim.close()
   return _baselines[key]
+
+
+def test_fields_are_the_float_model_fields(lib, go1):
+  """FIELDS plus the two arrays the kernel does not read are exactly the float model fields the library lists."""
+  import ctypes
+
+  from mjlab_b200.sim import native
+
+  sim = EmulSim(lib, go1, 1)
+  names = [lib.b2_field_name(sim.h, 1, i).decode() for i in range(lib.b2_num_fields(sim.h, 1))]
+  t = native.B2Tensor()
+  floats = []
+  for name in names:
+    assert lib.b2_get_field(sim.h, 1, name.encode(), ctypes.byref(t)) == 0
+    if t.dtype == 2:  # B2_F32
+      floats.append(name)
+  sim.close()
+  assert sorted(FIELDS + ["geom_rgba", "dof_frictionloss"]) == sorted(floats)
 
 
 @pytest.mark.parametrize("name", FIELDS)
